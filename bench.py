@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # our arm
     python bench.py --impl reference --gpus N --steps K ...    # reference CPU arm
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's logits to DIR
 
 Workload (BASELINE.json configs[1]): GNN inference, resize 128 pixel-grid graphs,
 batch 512 synthetic RGB images per GPU (weak scaling).  One "step" = graph build +
@@ -40,11 +41,24 @@ FWD_FLOP_PER_NODE = 525_568          # SURVEY.md 8d: fwd FLOPs per graph = 52556
 FWD_FLOP_PER_EDGE = 557_824
 
 
+def _count(least: int):
+    def integer(s: str) -> int:
+        v = int(s)
+        if v < least:
+            raise argparse.ArgumentTypeError(f"must be >= {least}, got {v}")
+        return v
+    return integer
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_count(1), default=5, help="timed steps of the headline inference step")
+    ap.add_argument("--warmup", type=_count(0), default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed inference step returned in its last step (logits, float32) as "
+                         "DIR/logits.npy (DIR/logits_rank<R>.npy per rank when there are several); the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared output for output")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--resize", type=int, default=128)
     ap.add_argument("--batch", type=int, default=512, help="graphs per GPU per step")
@@ -59,7 +73,10 @@ def parse_args():
     ap.add_argument("--power-seconds", type=float, default=3.0)
     ap.add_argument("--cpu-graphs", type=int, default=256, help="graphs in the bounded CPU sample")
     ap.add_argument("--ref-graphs-per-step", type=int, default=32)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of our arm's timed step; it does not apply to --impl reference")
+    return args
 
 
 def peaks():
@@ -94,6 +111,24 @@ def measured_traffic(key: str, sources):
     if not ent or ent.get("source_sha") != source_sha(*sources):
         return None, None
     return float(ent["dram_bytes_read"]) + float(ent["dram_bytes_write"]), ent.get("from")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict, suffix: str = "") -> None:
+    """Writes each tensor as ``out_dir/<name><suffix>.npy`` (float64 stays float64, everything else becomes float32)."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit; use a smaller --batch")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 class ClockSampler:
@@ -406,8 +441,8 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
     n_gpus = world
 
-    from graphnet_classifier_b200 import _lib, build, ops
-    build.build()
+    from graphnet_classifier_b200 import _lib, ops
+    _lib.load()         # the library build() made; the benchmark never compiles, so it runs from a read-only tree
     from graphnet_classifier_b200.models.GNN import CombinedModel, GraphNet
     from graphnet_classifier_b200.pipeline import GraphClassifierPipeline
     from graphnet_classifier_b200.utils.distributed import GradBucket, broadcast_parameters
@@ -458,8 +493,11 @@ def run_ours(args):
         return max_over_ranks(ms), wall
 
     # ---- inference, inputs resident in HBM (value) -------------------------------
+    last = {}
+
     def infer_step():
-        return pipe.infer(imgs_dev)
+        last["logits"] = pipe.infer(imgs_dev)
+        return last["logits"]
 
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -472,6 +510,8 @@ def run_ours(args):
     ms_total, wall = timed(infer_step, args.steps, 0)
     clocks = sampler.stop() if rank == 0 else None
     value = n_gpus * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": last["logits"]}, f"_rank{rank}" if world > 1 else "")
 
     # ---- board power under this step (outside every timed region) ---------------------------------------------------
     # The tensor-core launches of the path run AT the board's power cap (DESIGN.md section 5): the same step back to back
