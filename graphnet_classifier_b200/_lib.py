@@ -47,7 +47,8 @@ class GncTcChain(Structure):
                 ("narrow_W", c_void_p), ("ld_narrow_W", c_int64), ("narrow_b", c_void_p), ("narrow_k", c_int32), ("_pad2", c_int32),
                 ("stash_a1", c_void_p), ("stash_a2", c_void_p), ("stash_z", c_void_p), ("ld_stash", c_int64),
                 ("stash_mean", c_void_p), ("stash_rstd", c_void_p),
-                ("agg_rowptr", c_void_p), ("agg_eid", c_void_p)]
+                ("agg_rowptr", c_void_p), ("agg_eid", c_void_p),
+                ("edge_slots", c_int32), ("paired_operand", c_int32)]
 
 
 class GncBwdReduceItem(Structure):
@@ -104,6 +105,7 @@ SIGNATURES = {
     "gnc_gather_add_rows_f32": (c_int, [POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64), c_int, _P, c_int, c_int64,
                                         c_int, _P, c_int64, _P]),
     "gnc_grid_edge_class": (c_int, [c_int, c_int, c_int, c_int, _P, _P]),
+    "gnc_grid_pair_slots": (c_int, [c_int, c_int, c_int, _P, _P, _P, _P]),
     "gnc_edge_geometry_f32": (c_int, [_P, c_int, _P, _P, c_int64, _P, _P]),
     "gnc_linear_fwd_f32": (c_int, [POINTER(GncSeg), c_int, c_int64, _P, c_int64, _P, c_int, c_int, _P, c_int64, _P]),
     "gnc_linear_fwd_splitk_workspace": (c_int64, [c_int64, c_int, c_int64]),

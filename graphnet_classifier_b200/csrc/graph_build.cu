@@ -155,6 +155,19 @@ __global__ void grid_edge_class_kernel(GridDims g, int64_t BE, int32_t* __restri
   }
 }
 
+// paired destination slots of a batched grid graph without diagonals (grid_slot_src): for slot s of 2 B N, its source
+// node (-1: padding slot), its destination node s >> 1 and its edge class (0 horizontal, 1 vertical: the slot's parity)
+__global__ void grid_pair_slots_kernel(GridDims g, int64_t BS, int32_t* __restrict__ src, int32_t* __restrict__ dst,
+                                       int32_t* __restrict__ cls) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < BS; s += stride) {
+    const int64_t b = s / (2 * g.N), local = grid_slot_src(g, s - b * 2 * g.N);
+    src[s] = local < 0 ? -1 : (int32_t)(b * g.N + local);
+    dst[s] = (int32_t)(s >> 1);
+    cls[s] = (int32_t)(s & 1);
+  }
+}
+
 static int launch_grid_build(const uint8_t* img, int B, int imgH, int imgW, int patch, int diagonals,
                              float* x, float* pos, int64_t* ei, int32_t* src32, int32_t* dst32,
                              int32_t* drp, int32_t* deid, int32_t* srp, int32_t* seid, cudaStream_t st) {
@@ -688,6 +701,17 @@ int gnc_grid_edge_class(int B, int H, int W, int diagonals, int32_t* cls, gnc_st
   if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
   grid_edge_class_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(g, BE, cls);
   return check_launch("grid_edge_class_kernel");
+}
+
+int gnc_grid_pair_slots(int B, int H, int W, int32_t* slot_src, int32_t* slot_dst, int32_t* slot_class, gnc_stream_t stream) {
+  GNC_REQUIRE(B > 0 && H > 0 && W > 0 && slot_src && slot_dst && slot_class, "grid_pair_slots: bad arguments");
+  const GridDims g = make_grid(H, W, 0);
+  const int64_t BS = 2 * (int64_t)B * g.N;
+  GNC_REQUIRE(BS <= INT32_MAX, "grid_pair_slots: more than 2^31 slots");
+  int64_t blocks = ceil_div<int64_t>(BS, 256);
+  if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
+  grid_pair_slots_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(g, BS, slot_src, slot_dst, slot_class);
+  return check_launch("grid_pair_slots_kernel");
 }
 
 int64_t gnc_superpixel_workspace(int S_max, int max_label) {

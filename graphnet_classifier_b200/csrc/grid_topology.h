@@ -105,4 +105,23 @@ GNC_HD int grid_out_edges(const GridDims& g, int64_t v, int64_t ids[4], int64_t*
   return n;
 }
 
+// Paired destination slots (grids without diagonals, where a node has at most two in-edges).  Slot 2v holds the
+// horizontal in-edge of node v (from v-1, edge id i*(W-1)+j-1), slot 2v+1 the vertical one (from v-W, edge id
+// Eh+v-W): the slot order of the edge ids into v is their ascending order, so (0 + y[2v]) + y[2v+1] is
+// scatter_sum's bit pattern.  A slot whose edge does not exist (j = 0, resp. i = 0) is a padding slot.
+// Returns the local edge id held by slot s (0 <= s < 2N), or -1 for a padding slot.
+GNC_HD int64_t grid_slot_edge(const GridDims& g, int64_t s) {
+  const int W = g.W;
+  const int64_t v = s >> 1, i = v / W, j = v - i * W;
+  if ((s & 1) == 0) return j > 0 ? i * (W - 1) + (j - 1) : -1;
+  return i > 0 ? g.Eh + (v - W) : -1;
+}
+
+// Source node of slot s, or -1 for a padding slot.  The destination node of slot s is s >> 1.
+GNC_HD int64_t grid_slot_src(const GridDims& g, int64_t s) {
+  const int64_t v = s >> 1, i = v / g.W, j = v - i * g.W;
+  if ((s & 1) == 0) return j > 0 ? v - 1 : -1;
+  return i > 0 ? v - g.W : -1;
+}
+
 }  // namespace gnc

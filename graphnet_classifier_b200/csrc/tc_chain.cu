@@ -91,6 +91,9 @@ struct Params {
   // aggregated first operand (two-operand node form): A is the EDGE-row table and row m of the first operand is the ordered
   // sum of A[agg_eid[k]], k in [agg_rowptr[m], agg_rowptr[m + 1]) - at most two entries per row (caller-checked)
   const int32_t* agg_rowptr; const int32_t* agg_eid;
+  // paired destination slots (gnc_tc_chain_t): edge_slots 1 - a negative i0 marks a padding row (output +0.0), 2 - and Y
+  // takes the pair sums (0 + y[2v]) + y[2v + 1]; paired (node form) - row m of the first operand is (0 + A[2m]) + A[2m + 1]
+  int edge_slots; int paired;
   // training forward (two-tile kernel, Spec<1> / Spec<2>): a1, a2 (hidden ReLU outputs), z (LayerNorm input), row statistics
   float* st_a1; float* st_a2; float* st_z; long long ld_st; float* st_mean; float* st_rstd;
   long long num_tiles;
@@ -872,10 +875,14 @@ __device__ __forceinline__ void cp_async_wait_pending(int n) {
   }
 }
 
-template <int SPEC, bool STASH = false>
+template <int SPEC, bool STASH = false, bool PSUM = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chain2_kernel(const Params p) {
   // STASH (training forward): the hidden ReLU outputs, the LayerNorm input and the row statistics are written out as well
   static_assert(!STASH || !Spec<SPEC>::pre, "the stash belongs to the three-layer forms");
+  // Rows may be paired destination slots (p.edge_slots): a negative gather index i0 marks a padding slot, whose gathers
+  // read row 0 and whose output row is +0.0.  PSUM: the store emits node rows (0 + y[2v]) + y[2v + 1] instead of y -
+  // slots 2v, 2v + 1 are adjacent rows of the transpose tile, so the pair sum is formed where the stores are.
+  static_assert(!PSUM || !STASH, "the pair-sum output is an inference form");
   // kPre (Spec<7>): the first operand is built by the epilogue warps from three gathers (no loader, two MMA layers,
   // residual through a small table read directly); otherwise three MMA layers, residual rows = the tile's rows.
   constexpr bool kPre = Spec<SPEC>::pre;
@@ -1095,7 +1102,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       for (int i = 0; i < 4; ++i) {
         long long g = r0 + rl + 8 * i;
         g = g < p.M ? g : p.M - 1;
-        a0[i] = p.g0 + (has_i0 ? (long long)__ldg(p.i0 + g) : g) * p.ld_g0 + lane_col;
+        a0[i] = p.g0 + (has_i0 ? (long long)max(__ldg(p.i0 + g), 0) : g) * p.ld_g0 + lane_col;
         if (has_g1) a1[i] = p.g1 + (has_i1 ? (long long)__ldg(p.i1 + g) : g) * p.ld_g1 + lane_col;
       }
     };
@@ -1263,6 +1270,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
         if (S == 1 && !hasY) break;
         const long long row0 = tile_row0(2 * g + S);
         const bool tile_full = row0 + 32 <= p.M;
+        const bool pad_row = has_i0 && p.edge_slots && row0 + lane < p.M && __ldg(p.i0 + row0 + lane) < 0;
         if (!kPre && S == 0 && hasY) res_rows(jY);    // X's residual steps are all issued: the stream continues with Y's
         const float* rrow = nullptr;
         if (kPre) {
@@ -1342,18 +1350,35 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
             for (int jj = 0; jj < 16; ++jj) x[16 * c + jj] += rsd[jj];
             __syncwarp();
           }
+          if (pad_row) {
+#pragma unroll
+            for (int jj = 0; jj < 16; ++jj) x[16 * c + jj] = 0.f;
+          }
 #pragma unroll
           for (int ch = 0; ch < 4; ++ch)
             *reinterpret_cast<float4*>(slot + slot_off(lane, ch)) =
                 make_float4(x[16 * c + 4 * ch], x[16 * c + 4 * ch + 1], x[16 * c + 4 * ch + 2], x[16 * c + 4 * ch + 3]);
           __syncwarp();
-          float4 o[4];
+          if (PSUM) {                                               // node rows row0 / 2 + rl (+ 8): slot rows 2 rl, 2 rl + 1 (+ 16)
 #pragma unroll
-          for (int i = 0; i < 4; ++i) o[i] = *reinterpret_cast<const float4*>(slot + slot_off(rl + 8 * i, cc));
-          float* yrow = p.Y + (row0 + rl) * p.ldy + 32 * c + 16 * hf + 4 * cc;
+            for (int k = 0; k < 2; ++k) {
+              const int nr = rl + 8 * k;
+              const float4 a = *reinterpret_cast<const float4*>(slot + slot_off(2 * nr, cc));
+              const float4 b = *reinterpret_cast<const float4*>(slot + slot_off(2 * nr + 1, cc));
+              const float4 o = make_float4(__fadd_rn(__fadd_rn(0.f, a.x), b.x), __fadd_rn(__fadd_rn(0.f, a.y), b.y),
+                                           __fadd_rn(__fadd_rn(0.f, a.z), b.z), __fadd_rn(__fadd_rn(0.f, a.w), b.w));
+              if (tile_full || row0 + 2 * nr < p.M)
+                stg_hint(reinterpret_cast<float4*>(p.Y + ((row0 >> 1) + nr) * p.ldy + 32 * c + 16 * hf + 4 * cc), o, pol_drop);
+            }
+          } else {
+            float4 o[4];
 #pragma unroll
-          for (int i = 0; i < 4; ++i)
-            if (tile_full || row0 + rl + 8 * i < p.M) stg_hint(reinterpret_cast<float4*>(yrow + (long long)(8 * i) * p.ldy), o[i], pol_drop);
+            for (int i = 0; i < 4; ++i) o[i] = *reinterpret_cast<const float4*>(slot + slot_off(rl + 8 * i, cc));
+            float* yrow = p.Y + (row0 + rl) * p.ldy + 32 * c + 16 * hf + 4 * cc;
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+              if (tile_full || row0 + rl + 8 * i < p.M) stg_hint(reinterpret_cast<float4*>(yrow + (long long)(8 * i) * p.ldy), o[i], pol_drop);
+          }
           __syncwarp();
           // the slot is free again: next group of the stream
           if (!kPre && S == 0 && hasY) fetch_res(c);                // residual of Y, step c
@@ -1380,7 +1405,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 // the second operand into the same TMEM chunks once the first operand's MMAs have read them); RES: residual = the
 // tile's own rows of p.residual; TAIL 0: LayerNorm (if gamma) + residual -> Y, TAIL 1: relu . dot_w + dot_b.
 // Shared memory: (NL + K2) weight images, loader ring, two 2 KB slots per epilogue warp (residual ring / transpose).
-template <int NL, bool K2, bool RES, int TAIL, bool SYN = false, bool AGG = false>
+template <int NL, bool K2, bool RES, int TAIL, bool SYN = false, bool AGG = false, bool PAIR = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chain2n_kernel(const Params p) {
   static_assert(!(SYN && K2), "the synthesised operand is a single-operand form");
   // AGG: the first operand is not read but FORMED by the loader - row m = e[eid0] + e[eid1], the destination-ordered sum of
@@ -1389,6 +1414,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
   // edge row is read once, here.  Source 0 rides the cp.async ring (row addresses through the index), source 1 comes as
   // four 256-bit loads per chunk in the thread = row layout the ring is read back in.
   static_assert(!AGG || (K2 && NL == 3 && RES && TAIL == 0 && !SYN), "AGG belongs to the two-operand node form");
+  // PAIR (an AGG form): A is the paired destination slot table (gnc_grid_pair_slots) and row m's edge rows are the adjacent
+  // rows 2m, 2m + 1 (a zero row where an edge is missing) - the same two sources, with addresses instead of index lookups.
+  static_assert(!PAIR || AGG, "PAIR is a form of AGG");
   constexpr int kRegsLd = AGG ? 88 : kRegsLoader, kRegsEp = AGG ? 192 : kRegsEpi;
   static_assert(32 * (4 * kRegsLd + 4 * kRegsMma + kEpiWarps * kRegsEp) <= kThreads * 128, "setmaxnreg budget");
   constexpr int kImgs = NL + (K2 ? 1 : 0);
@@ -1518,12 +1546,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
     auto tile_row = [&](long long j) { return (pair + j * npairs) * kTileM + rank * 128 + q * 32 + lane; };
     auto load_rowptrs = [&](long long jx) {           // tiles jx, jx + 1
       rx0 = rx1 = ry0 = ry1 = 0;
-      if (!AGG) return;
+      if (!AGG || PAIR) return;
       if (jx < n_my) { const long long row = tile_row(jx); if (row < p.M) { rx0 = __ldg(p.agg_rowptr + row); rx1 = __ldg(p.agg_rowptr + row + 1); } }
       if (jx + 1 < n_my) { const long long row = tile_row(jx + 1); if (row < p.M) { ry0 = __ldg(p.agg_rowptr + row); ry1 = __ldg(p.agg_rowptr + row + 1); } }
     };
     auto load_eids = [&](long long jx) {              // tiles jx (even), jx + 1 from rx / ry
-      if (!AGG) return;
+      if (!AGG || PAIR) return;
       if (jx & 2) {
         ea2 = eb2 = ea3 = eb3 = -1;
         if (rx1 > rx0) ea2 = __ldg(p.agg_eid + rx0);
@@ -1547,9 +1575,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       long long j; int op, c;
       decode(it, j, op, c);
       if (op != 0) return;
-      const int e = ids_b(j);
-      if (e >= 0) {
-        const float* s2 = p.A + (long long)e * p.lda + c * 32;
+      const float* s2 = nullptr;
+      if (PAIR) {
+        const long long row = tile_row(j);
+        if (row < p.M) s2 = p.A + (2 * row + 1) * p.lda + c * 32;
+      } else {
+        const int e = ids_b(j);
+        if (e >= 0) s2 = p.A + (long long)e * p.lda + c * 32;
+      }
+      if (s2) {
 #pragma unroll
         for (int t = 0; t < 4; ++t) ldg256_stream(s2 + 8 * t, x2 + 8 * t);
       } else {
@@ -1566,7 +1600,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
         const float* src = op ? p.A2 : p.A;
         const long long ld = op ? p.lda2 : p.lda;
         const uint32_t dst0 = buf0 + (uint32_t)b * kChunkBytes;
-        if (AGG && op == 0) {
+        if (PAIR && op == 0) {                        // row m's first edge row: slot 2m
+          const float* s0 = src + 2 * row0 * ld + c * 32 + cj * 4;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const int r = i * 4 + rl;
+            const bool in = row0 + r < p.M;
+            cp_async16(dst0 + (uint32_t)(r * 128 + ((cj ^ (r & 7)) << 4)), in ? s0 + 2 * r * ld : src, in ? 16u : 0u);
+          }
+        } else if (AGG && op == 0) {
           const int mine = ids_a(j);
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
@@ -1632,7 +1674,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
           for (int jj = 0; jj < 4; ++jj) {
             float4 x = *reinterpret_cast<const float4*>(buf + (((half * 4 + jj) ^ (lane & 7)) << 4));
-            if (AGG && op == 0) {                     // (0 + a) + b: the ordered sum of the row's edges
+            if (PAIR && op == 0) {                    // (0 + a) + b, a = row 2m (horizontal), b = row 2m + 1 (vertical)
+              const float* y = x2 + 16 * half + 4 * jj;
+              x.x = __fadd_rn(__fadd_rn(0.f, x.x), y[0]); x.y = __fadd_rn(__fadd_rn(0.f, x.y), y[1]);
+              x.z = __fadd_rn(__fadd_rn(0.f, x.z), y[2]); x.w = __fadd_rn(__fadd_rn(0.f, x.w), y[3]);
+            } else if (AGG && op == 0) {              // (0 + a) + b: the ordered sum of the row's edges
               const float* y = x2 + 16 * half + 4 * jj;
               x.x += y[0]; x.y += y[1]; x.z += y[2]; x.w += y[3];
             }
@@ -1645,7 +1691,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       }
       // AGG: the last item of a group has been read back - its tiles' ids are dead, those of the group after the next
       // take their place (the copies of the next group's first items are already in flight with ids loaded a group ago)
-      if (AGG && op == kOps - 1 && c == 3 && (((j & 1) == 1) || j + 1 >= n_my)) {
+      if (AGG && !PAIR && op == kOps - 1 && c == 3 && (((j & 1) == 1) || j + 1 >= n_my)) {
         const long long jx = (j | 1) + 3;             // first tile of group g + 2 (g = this group)
         load_eids(jx);
         load_rowptrs(jx + 2);
@@ -1927,24 +1973,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
   }
 }
 
-template <int NL, bool K2, bool RES, int TAIL, bool SYN = false, bool AGG = false>
+template <int NL, bool K2, bool RES, int TAIL, bool SYN = false, bool AGG = false, bool PAIR = false>
 static int launch_spec2n(const Params& p, cudaStream_t st) {
   // (the kernel's own layout: weight images, loader ring, 2 slots per epilogue warp, constants, barriers, slack)
   constexpr int kSmem2n = (NL + (K2 ? 1 : 0)) * kLayerBytes + kLoaderWarps * kLoadBufs * kChunkBytes + kEpiWarps * 2 * kSlotBytes +
                           5 * kD * 4 + 2 * kEpiWarps * 32 * 4 + 320 + 1024;
   static SmemAttrOnce smem_attr;
-  if (int rc_attr = smem_attr.ensure(tc_chain2n_kernel<NL, K2, RES, TAIL, SYN, AGG>, kSmem2n, "tc_chain2n")) return rc_attr;
+  if (int rc_attr = smem_attr.ensure(tc_chain2n_kernel<NL, K2, RES, TAIL, SYN, AGG, PAIR>, kSmem2n, "tc_chain2n")) return rc_attr;
   long long pairs = p.num_tiles < kNumSMs / 2 ? p.num_tiles : kNumSMs / 2;
-  tc_chain2n_kernel<NL, K2, RES, TAIL, SYN, AGG><<<(unsigned)(2 * pairs), kThreads, kSmem2n, st>>>(p);
+  tc_chain2n_kernel<NL, K2, RES, TAIL, SYN, AGG, PAIR><<<(unsigned)(2 * pairs), kThreads, kSmem2n, st>>>(p);
   return check_launch("tc_chain2n_kernel");
 }
 
-template <int SPEC, bool STASH = false>
+template <int SPEC, bool STASH = false, bool PSUM = false>
 static int launch_spec2(const Params& p, cudaStream_t st) {
   static SmemAttrOnce smem_attr;
-  if (int rc_attr = smem_attr.ensure(tc_chain2_kernel<SPEC, STASH>, kSmemBytes, "tc_chain2")) return rc_attr;
+  if (int rc_attr = smem_attr.ensure(tc_chain2_kernel<SPEC, STASH, PSUM>, kSmemBytes, "tc_chain2")) return rc_attr;
   long long pairs = p.num_tiles < kNumSMs / 2 ? p.num_tiles : kNumSMs / 2;
-  tc_chain2_kernel<SPEC, STASH><<<(unsigned)(2 * pairs), kThreads, kSmemBytes, st>>>(p);
+  tc_chain2_kernel<SPEC, STASH, PSUM><<<(unsigned)(2 * pairs), kThreads, kSmemBytes, st>>>(p);
   return check_launch("tc_chain2_kernel");
 }
 
@@ -1963,10 +2009,15 @@ static int launch(const Params& p, cudaStream_t st) {
     return (p.g1 && p.i0) ? launch_spec2<1, true>(p, st) : launch_spec2<2, true>(p, st);
   }
   if (p.multi) return launch_spec<6>(p, st);
+  if (p.edge_slots) {                             // only the two-tile kernel knows padding slots (form validated by the caller)
+    if (!p.A) return p.edge_slots == 2 ? launch_spec2<7, false, true>(p, st) : launch_spec2<7>(p, st);
+    return p.edge_slots == 2 ? launch_spec2<1, false, true>(p, st) : launch_spec2<1>(p, st);
+  }
   if (!p.A) {
     static const bool two = []() { const char* e = getenv("GNC_CHAIN_TWO_TILES"); return !e || e[0] != '0'; }();
     return two ? launch_spec2<7>(p, st) : launch_spec<7>(p, st);
   }
+  if (p.A2 && p.paired) return launch_spec2n<3, true, true, 0, false, true, true>(p, st);
   if (p.A2 && p.agg_rowptr) return launch_spec2n<3, true, true, 0, false, true>(p, st);
   if (p.A2) return launch_spec2n<3, true, true, 0>(p, st);
   if (p.syn_W) return launch_spec2n<2, false, false, 0, true>(p, st);     // (shape validated by the caller)
@@ -2041,8 +2092,24 @@ extern "C" int gnc_tc_mlp_chain_f32(const float* A, int64_t lda, int64_t M, cons
                   "tc_mlp_chain: the aggregated operand needs agg_eid and 32-byte aligned edge rows (pitch a multiple of 8)");
       p.agg_rowptr = ch->agg_rowptr; p.agg_eid = ch->agg_eid;
     }
+    if (ch->paired_operand) {
+      GNC_REQUIRE(!ch->agg_rowptr && lda % 8 == 0 && ((uintptr_t)A) % 32 == 0,
+                  "tc_mlp_chain: the paired operand excludes agg_rowptr and needs 32-byte aligned slot rows (pitch a multiple of 8)");
+      p.paired = 1;
+    }
   } else {
-    GNC_REQUIRE(!ch->agg_rowptr, "tc_mlp_chain: agg_rowptr belongs to the two-operand form");
+    GNC_REQUIRE(!ch->agg_rowptr && !ch->paired_operand, "tc_mlp_chain: agg_rowptr / paired_operand belong to the two-operand form");
+  }
+  if (ch->edge_slots) {
+    // paired destination slots: the edge processor's two forms (three layers with gathers P[src], Q[dst], residual by row;
+    // or the pre-stage form of block 0)
+    GNC_REQUIRE(ch->edge_slots == 1 || ch->edge_slots == 2, "tc_mlp_chain: edge_slots is 0, 1 or 2");
+    GNC_REQUIRE(ch->gather0 && ch->gather0_idx && ch->gather1 && ch->gather1_idx && ch->gamma && ch->residual && !ch->dot_w &&
+                !ch->operand2 && !ch->narrow_W && !ch->stash_a1 &&
+                ((A && ch->nlayers == 3 && !ch->residual_idx) || (!A && ch->nlayers == 2)),
+                "tc_mlp_chain: edge_slots takes the edge processor's forms (two indexed gathers, LayerNorm, residual)");
+    GNC_REQUIRE(ch->edge_slots == 1 || M % 2 == 0, "tc_mlp_chain: pair sums need an even number of slot rows");
+    p.edge_slots = ch->edge_slots;
   }
   GNC_REQUIRE(ok4(ch->gather0, ch->ld_gather0) && ok4(ch->gather1, ch->ld_gather1) && ok4(ch->residual, ch->ld_residual),
               "tc_mlp_chain: addend / residual rows must be 16-byte aligned, 128 wide");

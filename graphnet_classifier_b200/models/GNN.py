@@ -230,13 +230,33 @@ class GraphNet(nn.Module):
         else:
             e = chain(ops.linear([ops.edge_geometry(pos, graph)], ee[0].weight, ee[0].bias, relu=True), None,
                       self.edge_encoder)
-        for blk in self.graph_processor.blocks:
+        # Grid graphs without diagonals (table form only): edge latents live in paired destination slots - slot 2v holds
+        # node v's horizontal in-edge, 2v + 1 its vertical one, a padding slot the row +0.0 - so scatter_sum(e, col) is
+        # (0 + e[2v]) + e[2v + 1] (the reference's order, bit for bit): two adjacent rows, no index.  The last block's edge
+        # launch writes these node sums instead of edge latents that nothing else reads.  A form of the aggregation folded
+        # into the node launch: GNC_FUSE_AGG=0 turns it off too.
+        slots = graph.pair_slots if (ops.PAIRED_EDGES and ops.FUSE_AGG and e is None) else None
+        blocks = self.graph_processor.blocks
+        for bi, blk in enumerate(blocks):
             em = blk.edge_model.edge_processor
             nm = blk.node_model.node_processor
             W0, b0 = em.model[0].weight, em.model[0].bias
             V0, c0 = nm.model[0].weight, nm.model[0].bias
             # the two node-side products of the edge processor read the same h: one launch
             P, Q = ops.tc_linear_multi(h, [W0[:, 0:128], W0[:, 128:256]])
+            if slots is not None:
+                s_src, s_dst, s_cls = slots
+                kw = dict(gather0=(P, s_src), gather1=(Q, s_dst), edge_slots=2 if bi == len(blocks) - 1 else 1)
+                if e is None:
+                    e = chain(None, None, em, pre=(tcl(e_tab, W0[:, 256:384]), s_cls, b0), residual=(e_tab, s_cls), **kw)
+                else:
+                    e = chain(e, (W0[:, 256:384], b0), em, residual=e, **kw)
+                del P, Q
+                if kw["edge_slots"] == 2:       # e holds the node sums: the plain two-operand form
+                    h = chain(e, (V0[:, 128:256], c0), nm, operand2=(h, V0[:, 0:128]), residual=h)
+                else:                           # the loader forms (0 + e[2m]) + e[2m + 1]
+                    h = chain(e, (V0[:, 128:256], c0), nm, operand2=(h, V0[:, 0:128]), residual=h, paired=True)
+                continue
             if e is None:       # block 0 in table form: e @ Wc.T is a 4-row table too
                 # relu(R[class] + P[row] + Q[col] + b0) is built inside the launch as its first operand
                 R = tcl(e_tab, W0[:, 256:384])

@@ -58,6 +58,10 @@ CHAIN_GUARD = os.environ.get("GNC_CHAIN_GUARD", "1") != "0"
 # scatter_sum folded into the node processor's launch when no node has more than two in-edges (grid graphs without
 # diagonals); "0" keeps the aggregation as a launch of its own (the form the fused one is tested against)
 FUSE_AGG = os.environ.get("GNC_FUSE_AGG", "1") != "0"
+# Inference on grid graphs without diagonals keeps edge latents in paired destination slots (GraphIndex.pair_slots): the
+# node launch reads a node's two edge rows as adjacent rows, and the last block's edge launch writes the per-node sums
+# instead of edge latents (with FUSE_AGG only).  "0" keeps edge-id order (the form the slot order is tested against).
+PAIRED_EDGES = os.environ.get("GNC_PAIRED_EDGES", "1") != "0"
 CHAIN_GUARD_EVENTS = 0          # how many forwards took the fallback (tests, diagnostics)
 
 
@@ -154,7 +158,8 @@ class GraphIndex:
     reference's summation order) and by source."""
 
     __slots__ = ("num_nodes", "num_edges", "src", "dst", "dst_rowptr", "dst_eid", "src_rowptr", "src_eid",
-                 "edge_class", "class_geom", "pos_ref", "pos_version", "class_sum_plan", "node_ptr", "_max_in_degree")
+                 "edge_class", "class_geom", "pos_ref", "pos_version", "class_sum_plan", "node_ptr", "_max_in_degree",
+                 "pair_slots")
 
     def __init__(self, num_nodes, num_edges, src, dst, dst_rowptr, dst_eid, src_rowptr, src_eid):
         self.num_nodes, self.num_edges = int(num_nodes), int(num_edges)
@@ -174,6 +179,10 @@ class GraphIndex:
         # fixed-size batches, where graph b owns rows b * num_nodes .. (b + 1) * num_nodes - 1
         self.node_ptr = None
         self._max_in_degree = None      # largest in-degree (lazy; builders that know it set it)
+        # Optional (grid builders, no diagonals): (src, dst, class) int32 [2 * num_nodes] of the paired destination slots -
+        # slot 2v holds node v's in-edge with the smaller edge id, slot 2v + 1 the other; src = -1 marks a slot without an
+        # edge (gnc_grid_pair_slots).  Edge latents in this row order need no index to be summed per node.
+        self.pair_slots = None
 
     def max_in_degree(self) -> int:
         """Largest number of edges arriving at one node: with at most two, the node processor's launch forms the
@@ -762,7 +771,7 @@ def tc_linear_multi(A: Tensor, weights: Sequence[Tensor], engine: str = "chain")
 def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1=None, gamma: Optional[Tensor] = None,
                  beta: Optional[Tensor] = None, eps: float = 1e-5, residual=None, dot_w: Optional[Tensor] = None,
                  dot_b: Optional[Tensor] = None, out: Optional[Tensor] = None, pre=None, operand2=None,
-                 narrow=None, stash=None, agg=None) -> Tensor:
+                 narrow=None, stash=None, agg=None, edge_slots: int = 0, paired: bool = False) -> Tensor:
     """Two or three chained ``Linear(128, 128)`` layers in one launch (csrc/tc_chain.cu), ReLU after
     all but the last, hidden activations kept on chip.  ``layers`` is ``[(W, bias), ...]``;
     ``gather0`` / ``gather1`` are ``(rows, idx int32 [M] | None)`` pre-activation addends of the first
@@ -775,6 +784,11 @@ def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1
     ``agg=(rowptr int32 [M + 1], eid int32)`` with ``operand2``: ``A`` is the ``[E, 128]`` edge table and the first operand's
     row ``m`` is the ordered sum of ``A[eid[k]]``, ``k`` in ``[rowptr[m], rowptr[m + 1])`` - at most two entries per row
     (``scatter_sum`` folded into the launch; the caller has checked the in-degrees).
+    ``edge_slots`` (edge processor forms; ``gather0`` / ``gather1`` indexed by ``GraphIndex.pair_slots``): 1 - the rows are
+    paired destination slots and a slot whose ``gather0`` index is negative gets the row +0.0; 2 - and the result is the
+    ``[M / 2, 128]`` per-node sum ``(0 + y[2v]) + y[2v + 1]`` instead of the slot rows.
+    ``paired=True`` with ``operand2``: ``A`` is the ``[2 M, 128]`` slot table and the first operand's row ``m`` is
+    ``(0 + A[2m]) + A[2m + 1]``.
     ``stash=(a1, a2, z, mean, rstd)`` (training forward of a block's edge / node MLP: 3 layers, addends, LayerNorm, residual
     by row): the launch also writes the hidden ReLU outputs ``a1``, ``a2``, the LayerNorm input ``z`` (``[M, 128]`` each) and
     the row statistics ``mean``, ``rstd`` (``[M]``) - what the backward pass of the MLP reads.
@@ -802,6 +816,11 @@ def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1
             M = rp.numel() - 1
             keep += [rp, ei]
             ch.agg_rowptr, ch.agg_eid = rp.data_ptr(), ei.data_ptr()
+        if paired:
+            if operand2 is None or agg is not None or M % 2 != 0:
+                raise ValueError("tc_mlp_chain: paired goes with operand2, without agg, on an even number of slot rows")
+            M //= 2
+            ch.paired_operand = 1
         a_ptr, a_ld, dev = A.data_ptr(), _ld(A), A.device
         if narrow is not None:
             Wn, bn = narrow
@@ -821,7 +840,7 @@ def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1
         keep.append(W)
         ch.W[l], ch.ldw[l] = W.data_ptr(), W.stride(0)
         ch.bias[l] = None if b is None else b.data_ptr()
-    nbytes = 4.0 * (((A.shape[0] if agg is not None else M) * (A.shape[1] if narrow is not None else 128) if A is not None else 0)
+    nbytes = 4.0 * (((A.shape[0] if (agg is not None or paired) else M) * (A.shape[1] if narrow is not None else 128) if A is not None else 0)
                     + len(layers) * 128 * 128 + (2 * M + 1 if agg is not None else 0))
     if operand2 is not None:
         A2, W2 = operand2
@@ -857,7 +876,13 @@ def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1
             t = rows(residual)
             ch.residual, ch.ld_residual = t.data_ptr(), _ld(t)
         nbytes += 4.0 * t.shape[0] * 128
-    n_out = 128
+    n_out, m_out = 128, M
+    if edge_slots:
+        if edge_slots not in (1, 2) or (edge_slots == 2 and M % 2 != 0):
+            raise ValueError("tc_mlp_chain: edge_slots is 1, or 2 on an even number of slot rows")
+        ch.edge_slots = int(edge_slots)
+        if edge_slots == 2:
+            m_out = M // 2
     if dot_w is not None:
         dw = dot_w.reshape(-1)
         if dw.stride(0) != 1:
@@ -867,8 +892,8 @@ def tc_mlp_chain(A: Optional[Tensor], layers: Sequence, *, gather0=None, gather1
         ch.dot_b = None if dot_b is None else dot_b.data_ptr()
         n_out = 1
     if out is None:
-        out = torch.empty(M, n_out, dtype=torch.float32, device=dev)
-    nbytes += 4.0 * M * n_out
+        out = torch.empty(m_out, n_out, dtype=torch.float32, device=dev)
+    nbytes += 4.0 * m_out * n_out
     if stash is not None:
         a1s, a2s, zs, means, rstds = stash
         for t in (a1s, a2s, zs):

@@ -130,6 +130,12 @@ def _build_grid(images, patch: int, diagonals: bool, device, use_cache: bool) ->
                     geom[c, 2] = rel.abs().sum()
             graph.edge_class, graph.class_geom = cls, geom
             graph.bind_positions(pos)
+            if not (diagonals and not patch):
+                # at most two in-edges per node: paired destination slots for the inference path (GraphIndex.pair_slots)
+                slots = torch.empty(3, 2 * B * N, dtype=torch.int32, device=dev)
+                check(lib.gnc_grid_pair_slots(B, gh, gw, slots[0].data_ptr(), slots[1].data_ptr(), slots[2].data_ptr(),
+                                              _stream()), "grid_pair_slots")
+                graph.pair_slots = (slots[0], slots[1], slots[2])
         attach_graph(ei, graph)
         if use_cache:
             _topology_cache.put(key, (pos, ei, graph))

@@ -247,6 +247,10 @@ int gnc_gather_add_rows_f32(const float* const* tables /*HOST*/, const int32_t* 
 /* Edge family of a batched H x W grid graph (0 horizontal, 1 vertical, 2/3 diagonals): all edges of
  * a family share one geometry row (models/GNN.py:299-302 applied to grid positions).  cls int32 [B*E]. */
 int gnc_grid_edge_class(int B, int H, int W, int diagonals, int32_t* cls, gnc_stream_t stream);
+/* Paired destination slots of a batch of B grids H x W without diagonals (csrc/grid_topology.h): 2 B H W slots, slot 2v
+ * for the horizontal in-edge of node v, 2v + 1 for the vertical one.  Writes each slot's source node (-1: no such edge,
+ * a padding slot), destination node (s >> 1) and edge class (0 / 1), int32 [2 B H W] each. */
+int gnc_grid_pair_slots(int B, int H, int W, int32_t* slot_src, int32_t* slot_dst, int32_t* slot_class, gnc_stream_t stream);
 
 /* edge_attr[e] = [pos[dst[e]] - pos[src[e]], sum |.|]  (models/GNN.py:299-302).
  * pos float [N, P]; out float [E, P+1]; 1 <= P <= 8. */
@@ -401,6 +405,14 @@ typedef struct gnc_tc_chain {
    * of NODE rows; agg_rowptr is int32 [M + 1]; every row must have AT MOST TWO entries (the caller checks the topology once:
    * grid graphs without diagonals) - with those the sum is the reference's bit for bit. */
   const int32_t* agg_rowptr; const int32_t* agg_eid;
+  /* paired destination slots (gnc_grid_pair_slots; grids without diagonals, at most two in-edges per node).
+   * edge_slots = 1 (the three-layer edge form with two indexed gathers, or the pre-stage form): the M rows are slots, and a
+   *   NEGATIVE gather0_idx marks a padding slot - its gathers read row 0 and its output row is exactly +0.0.
+   * edge_slots = 2: as 1, and Y gets M / 2 node rows (M even) Y[v] = (0 + y[2v]) + y[2v + 1] instead of the M slot rows y -
+   *   scatter_sum(edge_attr, col) of the next node processor, in the reference's order, with no [M, 128] edge output.
+   * paired_operand = 1 (the two-operand node form, without agg_rowptr): A is the [2M, 128] slot table and row m of the
+   *   first operand is (0 + A[2m]) + A[2m + 1]. */
+  int32_t edge_slots; int32_t paired_operand;
 } gnc_tc_chain_t;
 
 int gnc_tc_mlp_chain_f32(const float* A, int64_t lda, int64_t M, const gnc_tc_chain_t* chain /*HOST*/,
