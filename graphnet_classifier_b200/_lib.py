@@ -155,6 +155,8 @@ SIGNATURES = {
     "gnc_debug_slic_connect_streaming": (c_int, [c_int]),
     "gnc_superpixel_batch_offsets": (c_int, [_P, _P, c_int, c_int, c_int64, _P, _P, _P]),
     "gnc_superpixel_batch_compact": (c_int, [_P, _P, _P, c_int, c_int, c_int64, _P, _P, _P, _P, _P, c_int64, _P]),
+    "gnc_superpixel_batch_padded": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int64, _P, _P,
+                                            _P, _P, _P, _P, _P]),
     "gnc_jpeg_parse": (c_int, [_P, c_int64, POINTER(GncJpegImage)]),
     "gnc_jpeg_pack": (c_int, [_P, _P, c_int, c_int, _P, c_int64, _P, _P, _P]),
     "gnc_jpeg_scratch_bytes": (c_int64, [c_int64, c_int]),

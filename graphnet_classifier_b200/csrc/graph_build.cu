@@ -10,6 +10,8 @@
 //   utils/dataloader.py:49-51 (casts to float32 / float32 / int64)
 #include <stdlib.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "grid_topology.h"
 
@@ -661,6 +663,57 @@ __global__ void __launch_bounds__(256) superpixel_compact_kernel(const float* __
   }
 }
 
+// The same batch at host-known sizes (N_alloc = B * S_cap + 1 rows, E_alloc = B * E_cap edges), so that nothing has to
+// be read back and the build can be captured in a CUDA graph.  Rows [0, node_ptr[B]) and edges [0, edge_ptr[B]) are what
+// superpixel_compact_kernel writes.  The padding rows [P0, N_alloc) are zero and padding edge P0 + k is a self-loop of
+// padding row P0 + k mod (N_alloc - P0): no real row meets a padding edge, and the padding rows' in-degrees stay near
+// E_pad / N_pad, which keeps the CSR build's per-row sort and the aggregation's per-row loop short.  Every offset is
+// clamped to the buffers, so nothing is written out of bounds whatever the inputs hold; what does not fit is reported
+// in *overflow (bit 0: a label outside [0, max_label], bit 1: more than S_cap nodes, bit 2: more than E_cap edges).
+__global__ void __launch_bounds__(256) superpixel_padded_kernel(
+    const float* __restrict__ x, const float* __restrict__ pos, const int64_t* __restrict__ edges,
+    const int32_t* __restrict__ n_nodes, const int32_t* __restrict__ n_edges, const int32_t* __restrict__ labels,
+    int B, int64_t HW, int max_label, int S_cap, int64_t E_cap, const int32_t* __restrict__ node_ptr,
+    const int64_t* __restrict__ edge_ptr, float* __restrict__ xb, float* __restrict__ pb, int64_t* __restrict__ eb,
+    int32_t* __restrict__ overflow) {
+  const int64_t N_alloc = (int64_t)B * S_cap + 1, E_alloc = (int64_t)B * E_cap;
+  auto clamp = [](int64_t v, int64_t lo, int64_t hi) { return v < lo ? lo : (v > hi ? hi : v); };
+  int bad = 0;
+  for (int b = blockIdx.x; b < B; b += gridDim.x) {
+    if (n_nodes[b] > S_cap) bad |= 2;
+    if (n_edges[b] > E_cap) bad |= 4;
+    const int64_t n0 = clamp(node_ptr[b], 0, N_alloc - 1);
+    const int64_t nn = clamp((int64_t)node_ptr[b + 1] - node_ptr[b], 0, S_cap < N_alloc - 1 - n0 ? S_cap : N_alloc - 1 - n0);
+    const int64_t e0 = clamp(edge_ptr[b], 0, E_alloc);
+    const int64_t ne = clamp(edge_ptr[b + 1] - edge_ptr[b], 0, E_cap < E_alloc - e0 ? E_cap : E_alloc - e0);
+    const float* xs = x + (int64_t)b * S_cap * 3;
+    const float* ps = pos + (int64_t)b * S_cap * 2;
+    for (int64_t i = threadIdx.x; i < nn * 3; i += blockDim.x) xb[n0 * 3 + i] = xs[i];
+    for (int64_t i = threadIdx.x; i < nn * 2; i += blockDim.x) pb[n0 * 2 + i] = ps[i];
+    const int64_t* es = edges + (int64_t)b * 2 * E_cap;
+    for (int64_t i = threadIdx.x; i < ne; i += blockDim.x) {
+      eb[e0 + i] = es[i] + n0;
+      eb[E_alloc + e0 + i] = es[E_cap + i] + n0;
+    }
+  }
+  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nthreads = (int64_t)gridDim.x * blockDim.x;
+  const int64_t P0 = clamp(node_ptr[B], 0, N_alloc - 1), Q0 = clamp(edge_ptr[B], 0, E_alloc);
+  for (int64_t i = P0 * 3 + tid; i < N_alloc * 3; i += nthreads) xb[i] = 0.f;
+  for (int64_t i = P0 * 2 + tid; i < N_alloc * 2; i += nthreads) pb[i] = 0.f;
+  for (int64_t k = Q0 + tid; k < E_alloc; k += nthreads) {
+    const int64_t v = P0 + (k - Q0) % (N_alloc - P0);
+    eb[k] = v;
+    eb[E_alloc + k] = v;
+  }
+  if (labels) {
+    for (int64_t p = tid; p < (int64_t)B * HW; p += nthreads) {
+      const int32_t l = labels[p];
+      if (l < 0 || l > max_label) bad |= 1;
+    }
+  }
+  if (bad) atomicOr(overflow, bad);
+}
+
 }  // namespace gnc
 
 using namespace gnc;
@@ -758,6 +811,26 @@ int gnc_superpixel_batch_compact(const float* x, const float* pos, const int64_t
               e_total >= 0, "superpixel_batch_compact: bad arguments");
   superpixel_compact_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(x, pos, edges, S_max, E_max, node_ptr, edge_ptr, xb, pb, eb, e_total);
   return check_launch("superpixel_compact_kernel");
+}
+
+int gnc_superpixel_batch_padded(const float* x, const float* pos, const int64_t* edges, const int32_t* n_nodes,
+                                const int32_t* n_edges, const int32_t* labels, int B, int H, int W, int max_label,
+                                int S_cap, int64_t E_cap, const int32_t* node_ptr, const int64_t* edge_ptr, float* xb,
+                                float* pb, int64_t* eb, int32_t* overflow, gnc_stream_t stream) {
+  GNC_REQUIRE(x && pos && edges && n_nodes && n_edges && node_ptr && edge_ptr && xb && pb && overflow && B > 0 && S_cap > 0 &&
+              E_cap >= 0 && (eb || E_cap == 0) && (!labels || (H > 0 && W > 0 && max_label >= 0)),
+              "superpixel_batch_padded: bad arguments");
+  GNC_REQUIRE((int64_t)B * S_cap + 1 < INT32_MAX && (int64_t)B * E_cap < INT32_MAX,
+              "superpixel_batch_padded: node and edge counts must fit int32");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(overflow, 0, sizeof(int32_t), st);
+  if (e != cudaSuccess) return fail(GNC_ECUDA, "superpixel_batch_padded memset: %s", cudaGetErrorString(e));
+  const int64_t HW = labels ? (int64_t)H * W : 0;
+  const int64_t work = (int64_t)B * (HW + E_cap + 3 * S_cap);
+  const int64_t blocks = std::max<int64_t>(B, std::min<int64_t>(ceil_div<int64_t>(work, 256 * 8), (int64_t)kNumSMs * 4));
+  superpixel_padded_kernel<<<(unsigned)blocks, 256, 0, st>>>(x, pos, edges, n_nodes, n_edges, labels, B, HW, max_label, S_cap,
+                                                              E_cap, node_ptr, edge_ptr, xb, pb, eb, overflow);
+  return check_launch("superpixel_padded_kernel");
 }
 
 int64_t gnc_csr_workspace(int64_t N) { return N + (N + 1) / 1024 + 64; }

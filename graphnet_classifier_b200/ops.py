@@ -63,6 +63,9 @@ FUSE_AGG = os.environ.get("GNC_FUSE_AGG", "1") != "0"
 # instead of edge latents (with FUSE_AGG only).  "0" keeps edge-id order (the form the slot order is tested against).
 PAIRED_EDGES = os.environ.get("GNC_PAIRED_EDGES", "1") != "0"
 CHAIN_GUARD_EVENTS = 0          # how many forwards took the fallback (tests, diagnostics)
+# how many GraphClassifierPipeline.infer_graphed calls on superpixel graphs found a label map beyond the captured
+# batch's capacities and returned the exact builder's logits instead (tests, diagnostics)
+SUPERPIXEL_OVERFLOW_EVENTS = 0
 
 
 def _require_cuda(*ts: Tensor) -> None:

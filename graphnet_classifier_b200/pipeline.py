@@ -3,6 +3,10 @@
     pipe = GraphClassifierPipeline(model, resize_value=128)
     logits = pipe.infer(images_u8)                      # [B, classes]
     loss = pipe.train_step(images_u8, labels, optimizer)
+    pipe = GraphClassifierPipeline(model, 256, method="superpixel", n_segments=100, compactness=10.0)
+
+``method``: "pixel" / "patch" grid graphs, or "superpixel" graphs of the device SLIC labels (one node per region,
+graphs of different node counts in one block-diagonal batch; the model's readout pads / truncates per graph).
 
 ``images_u8`` is ``uint8 [B, r, r, 3]`` on the host (pinned or not) or on the device.
 Per call: one host->device copy of the pixels (if needed), the fused graph-build
@@ -21,29 +25,43 @@ import torch
 from torch import Tensor
 
 from . import ops
-from .utils.image_to_graph.batched import build_patch_graphs, build_pixel_graphs
+from .utils.image_to_graph.batched import (build_patch_graphs, build_pixel_graphs, build_superpixel_batch,
+                                           build_superpixel_batch_padded, superpixel_capacity)
+from .utils.image_to_graph.slic import connectivity_min_size, slic_labels
 
 
 class GraphClassifierPipeline:
     def __init__(self, model: torch.nn.Module, resize_value: int, diagonals: bool = False, method: str = "pixel",
                  patch_size: int = 8, micro_batch: Optional[int] = None, train_micro_batch: Optional[int] = None,
-                 device=None):
+                 device=None, n_segments: int = 100, compactness: float = 10.0):
         self.model = model
         self.resize_value = int(resize_value)
         self.diagonals = bool(diagonals)
         self.method = method
         self.patch_size = int(patch_size)
+        # superpixel graphs: the reference's slic(image, n_segments=100, compactness=10) (image_to_graph_superpixel.py:31)
+        self.n_segments = int(n_segments)
+        self.compactness = float(compactness)
         self.device = torch.device(device) if device is not None else next(model.parameters()).device
         if self.device.type != "cuda":
             raise RuntimeError("GraphClassifierPipeline needs the model on a CUDA device (no CPU fallback)")
-        n = self.resize_value * self.resize_value if method == "pixel" else (self.resize_value // self.patch_size) ** 2
+        r = self.resize_value
+        if method == "superpixel":
+            # per-image node / edge capacities of the captured path (superpixel_capacity); E <= 6 S, three times a
+            # grid node's share of edge rows, so a superpixel node is budgeted as three grid nodes
+            self.superpixel_caps = superpixel_capacity(r, r, connectivity_min_size(r, r, self.n_segments))
+            n = 3 * self.superpixel_caps[0]
+        else:
+            self.superpixel_caps = None
+            n = r * r if method == "pixel" else (r // self.patch_size) ** 2
         # live fp32 activations: ~8 KB per node in inference (5 edge tensors + node tensors of
         # width 128, E ~ 2N); training peaks at ~24 KB per node (activations kept for the backward over 3 blocks plus
         # the backward's transients: 63.6 GiB measured for 171 resize-128 graphs); budget 64 GiB of the 180 GB for
-        # inference and 100 GiB for training (256 resize-128 graphs per micro-batch: two per 512-graph step)
-        self.micro_batch = micro_batch or max(1, min(512, (64 << 30) // (n * 8192)))
+        # inference and 100 GiB for training (256 resize-128 graphs per micro-batch: two per 512-graph step).
+        # Superpixel graphs are small (~100 nodes): up to 1024 per call, config 4's batch in one build.
+        self.micro_batch = micro_batch or max(1, min(1024 if method == "superpixel" else 512, (64 << 30) // (n * 8192)))
         self.train_micro_batch = train_micro_batch or max(1, min(256, (100 << 30) // (n * 24_000)))
-        self._graphs = {}            # image batch shape -> (CUDAGraph, static input, static logits)
+        self._graphs = {}            # capture key -> (CUDAGraph, static input, static logits, static overflow flag)
 
     # -- staging ----------------------------------------------------------------
     def _to_device(self, images) -> Tensor:
@@ -68,7 +86,20 @@ class GraphClassifierPipeline:
             return build_pixel_graphs(images_dev, diagonals=self.diagonals)
         if self.method == "patch":
             return build_patch_graphs(images_dev, patch_size=self.patch_size)
+        if self.method == "superpixel":
+            return build_superpixel_batch(images_dev, labels=self._labels(images_dev))
         raise ValueError(f"Unknown method: {self.method}")
+
+    def _labels(self, images_dev: Tensor) -> Tensor:
+        return slic_labels(images_dev, n_segments=self.n_segments, compactness=self.compactness)
+
+    def _build_captured(self, images_dev: Tensor):
+        """The graph build of ``infer_graphed``: ``(GraphBatch, overflow flag or None)``.  Superpixel batches take the
+        padded builder there, whose sizes are known on the host; the exact one reads its output sizes back."""
+        if self.method != "superpixel":
+            return self._build(images_dev), None
+        S_cap, E_cap = self.superpixel_caps
+        return build_superpixel_batch_padded(images_dev, self._labels(images_dev), S_cap, E_cap)
 
     @staticmethod
     def _even_chunk(total: int, limit: int) -> int:
@@ -96,20 +127,27 @@ class GraphClassifierPipeline:
         (utils/inference.py:32-71).  The whole call (graph build, GraphNet, head: ~25 launches) is
         captured once per batch shape as a CUDA graph and replayed; the pixels are copied into the
         graph's static input.  Same kernels, same results as ``infer``; the model's parameters are
-        read at replay time, so updated weights are picked up, a changed architecture is not."""
+        read at replay time, so updated weights are picked up, a changed architecture is not.
+
+        Superpixel graphs (SLIC, connectivity pass, graph kernel, padded batch, CSR, GraphNet, readout and head in
+        one graph) are built at the per-image capacities ``superpixel_caps``, which the pipeline's own labels cannot
+        exceed; the logits are ``infer``'s, bit for bit.  This call ends in one synchronisation: it reads the
+        capacity flag back.  Should it be set, the call returns ``infer(images)`` instead and counts the event in
+        ``ops.SUPERPIXEL_OVERFLOW_EVENTS``."""
         t = images if isinstance(images, Tensor) else torch.as_tensor(images)
         if t.dim() == 3:
             t = t.unsqueeze(0)
-        key = tuple(t.shape)
+        key = (tuple(t.shape), self.superpixel_caps)
         ent = self._graphs.get(key)
         if ent is None:
             if t.shape[0] > self.micro_batch:
                 raise ValueError("infer_graphed is the small-batch path: use infer() for large batches")
-            static_in = torch.zeros(key, dtype=torch.uint8, device=self.device)
+            static_in = torch.zeros(key[0], dtype=torch.uint8, device=self.device)
 
             def run():
-                out = self.model(self._build(static_in).as_tuple())
-                return out.reshape(1, -1) if out.dim() == 1 else out
+                gb, flag = self._build_captured(static_in)
+                out = self.model(gb.as_tuple())
+                return (out.reshape(1, -1) if out.dim() == 1 else out), flag
 
             side = torch.cuda.Stream(device=self.device)
             side.wait_stream(torch.cuda.current_stream(self.device))
@@ -119,12 +157,18 @@ class GraphClassifierPipeline:
             torch.cuda.current_stream(self.device).wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                static_out = run()
-            ent = self._graphs[key] = (graph, static_in, static_out)
-        graph, static_in, static_out = ent
+                static_out, static_flag = run()
+            ent = self._graphs[key] = (graph, static_in, static_out, static_flag)
+        graph, static_in, static_out, static_flag = ent
         static_in.copy_(t, non_blocking=True)
         graph.replay()
-        return static_out.clone()
+        out = static_out.clone()
+        if static_flag is not None and int(static_flag.item()) != 0:
+            # a label map the capacities do not cover (cannot happen with the pipeline's own SLIC labels unless the
+            # bound's derivation is wrong): the exact builder, same logits
+            ops.SUPERPIXEL_OVERFLOW_EVENTS += 1
+            return self.infer(t)
+        return out
 
     # -- training -----------------------------------------------------------------
     def forward_backward(self, images, labels) -> Tensor:

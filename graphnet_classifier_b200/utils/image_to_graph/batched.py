@@ -226,3 +226,74 @@ def build_superpixel_batch(images, labels=None, n_segments: int = 100, compactne
     graph.node_ptr = node_ptr
     attach_graph(eb, graph)
     return GraphBatch(xb, pb, eb, graph, B, 0)
+
+
+def superpixel_capacity(H: int, W: int, min_size: int):
+    """Per-image ``(S_cap, E_cap)``: node and directed-edge bounds of the superpixel graphs of ``slic_labels`` maps whose
+    connectivity post-pass ran with ``min_size`` (``slic.connectivity_min_size``).
+
+    Nodes: the post-pass (csrc/slic_connect.cu) keeps a 4-connected component only if it has at least ``min_size``
+    pixels, except the component of pixel 0, which it always keeps; the kept components are the final labels.  Disjoint
+    components of ``min_size`` pixels or more number at most ``H W // min_size``, so ``S <= H W // min_size + 1``, and
+    ``S <= H W`` always (every component survives when ``min_size <= 1``).
+    Edges: every final label is a 4-connected region (a dissolved component joins the component next to its first pixel),
+    so contracting the regions of the pixel grid gives the region adjacency graph as a minor of a planar graph: it is
+    planar and simple, with at most ``3 S - 6`` adjacent pairs (``S >= 3``), i.e. ``6 S - 12`` directed edges; with
+    ``S < 3`` at most ``S (S - 1)``."""
+    hw = int(H) * int(W)
+    S = min(hw, hw // max(int(min_size), 1) + 1)
+    return S, (S * (S - 1) if S < 3 else 6 * S - 12)
+
+
+def build_superpixel_batch_padded(images, labels, S_cap: int, E_cap: int, device=None):
+    """``build_superpixel_batch`` at host-known sizes, for CUDA-graph capture: no value is read back to the host.
+
+    Returns ``(GraphBatch, overflow)``.  The batch has ``B S_cap + 1`` rows and ``B E_cap`` edges; its first
+    ``node_ptr[B]`` rows and ``edge_ptr[B]`` edges are ``build_superpixel_batch``'s, in the same order; the rest are zero
+    rows and self-loops on them (``gnc_superpixel_batch_padded``).  ``graph.node_ptr`` is the exact per-graph offsets,
+    so the readout sees the real rows only; every real node has the same in-edges, in the same order, as in the exact
+    batch, so the logits are the same bits.  ``overflow`` (int32 ``[1]`` on the device) is non-zero when an image has
+    a label outside ``[0, S_cap - 1]``, more than ``S_cap`` nodes or more than ``E_cap`` edges: the batch is then not
+    the exact one and its logits must not be used."""
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    img = _as_device_u8(images, dev)
+    lab = labels if isinstance(labels, Tensor) else torch.as_tensor(labels)
+    if lab.dim() == 2:
+        lab = lab.unsqueeze(0)
+    B, H, W, _ = img.shape
+    if tuple(lab.shape) != (B, H, W):
+        raise ValueError(f"labels must be [B, H, W] = {(B, H, W)}, got {tuple(lab.shape)}")
+    S_cap, E_cap = int(S_cap), int(E_cap)
+    if S_cap < 1 or E_cap < 0:
+        raise ValueError("S_cap must be >= 1 and E_cap >= 0")
+    lab32 = lab.to(dev, torch.int32).contiguous()
+    max_label = S_cap - 1                  # labels above it are skipped by the graph kernel and flagged below
+    lib = _lib.load()
+    i32 = dict(dtype=torch.int32, device=dev)
+    n_nodes, n_edges = torch.empty(B, **i32), torch.empty(B, **i32)
+    x = torch.empty(B, S_cap, 3, dtype=torch.float32, device=dev)
+    pos = torch.empty(B, S_cap, 2, dtype=torch.float32, device=dev)
+    adj = torch.empty(B, S_cap, S_cap, dtype=torch.uint8, device=dev)
+    edges = torch.empty(B, 2, max(E_cap, 1), dtype=torch.int64, device=dev)
+    work = _workspace(dev, B * int(lib.gnc_superpixel_workspace(S_cap, max_label)), torch.int32)
+    check(lib.gnc_build_superpixel_graph(img.data_ptr(), lab32.data_ptr(), B, H, W, max_label, S_cap, E_cap,
+                                         n_nodes.data_ptr(), x.data_ptr(), pos.data_ptr(), adj.data_ptr(),
+                                         n_edges.data_ptr(), edges.data_ptr(), work.data_ptr(), _stream()),
+          "build_superpixel_graph")
+    node_ptr = torch.empty(B + 1, **i32)
+    edge_ptr = torch.empty(B + 1, dtype=torch.int64, device=dev)
+    check(lib.gnc_superpixel_batch_offsets(n_nodes.data_ptr(), n_edges.data_ptr(), B, S_cap, E_cap, node_ptr.data_ptr(),
+                                           edge_ptr.data_ptr(), _stream()), "superpixel_batch_offsets")
+    N_alloc, E_alloc = B * S_cap + 1, B * E_cap
+    xb = torch.empty(N_alloc, 3, dtype=torch.float32, device=dev)
+    pb = torch.empty(N_alloc, 2, dtype=torch.float32, device=dev)
+    eb = torch.empty(2, max(E_alloc, 1), dtype=torch.int64, device=dev)[:, :E_alloc]
+    overflow = torch.empty(1, **i32)
+    check(lib.gnc_superpixel_batch_padded(x.data_ptr(), pos.data_ptr(), edges.data_ptr(), n_nodes.data_ptr(),
+                                          n_edges.data_ptr(), lab32.data_ptr(), B, H, W, max_label, S_cap, E_cap,
+                                          node_ptr.data_ptr(), edge_ptr.data_ptr(), xb.data_ptr(), pb.data_ptr(),
+                                          eb.data_ptr(), overflow.data_ptr(), _stream()), "superpixel_batch_padded")
+    graph = GraphIndex.from_edge_index(eb, N_alloc, validate=False)      # every endpoint is in range by construction
+    graph.node_ptr = node_ptr
+    attach_graph(eb, graph)
+    return GraphBatch(xb, pb, eb, graph, B, 0), overflow

@@ -32,6 +32,12 @@ def enforce_connectivity(labels: Tensor, min_size: int) -> Tensor:
     return out
 
 
+def connectivity_min_size(H: int, W: int, n_segments: int, min_size_factor: float = 0.5) -> int:
+    """``min_size`` of the connectivity post-pass of ``slic_labels``: ``int(min_size_factor * H * W / n_centres)``."""
+    n_centres = int(_lib.load().gnc_slic_num_centers(int(H), int(W), int(n_segments)))
+    return int(min_size_factor * H * W / max(n_centres, 1))
+
+
 def slic_labels(images: Tensor, n_segments: int = 100, compactness: float = 10.0, max_num_iter: int = 10,
                 enforce_connectivity_: bool = True, min_size_factor: float = 0.5) -> Tensor:
     """uint8 ``[B, H, W, 3]`` (or ``[H, W, 3]``) on the device -> int32 labels ``[B, H, W]``.  As scikit-image's
@@ -50,6 +56,5 @@ def slic_labels(images: Tensor, n_segments: int = 100, compactness: float = 10.0
     check(lib.gnc_slic_labels_u8(img.data_ptr(), B, H, W, int(n_segments), float(compactness), int(max_num_iter),
                                  labels.data_ptr(), work.data_ptr(), _stream()), "slic_labels")
     if enforce_connectivity_:
-        n_centres = int(lib.gnc_slic_num_centers(H, W, int(n_segments)))
-        labels = enforce_connectivity(labels, int(min_size_factor * H * W / max(n_centres, 1)))
+        labels = enforce_connectivity(labels, connectivity_min_size(H, W, n_segments, min_size_factor))
     return labels

@@ -119,6 +119,19 @@ int gnc_superpixel_batch_offsets(const int32_t* n_nodes, const int32_t* n_edges,
 int gnc_superpixel_batch_compact(const float* x, const float* pos, const int64_t* edges, int B, int S_max, int64_t E_max,
                                  const int32_t* node_ptr, const int64_t* edge_ptr, float* xb, float* pb, int64_t* eb,
                                  int64_t e_total, gnc_stream_t stream);
+/* The same batch at host-known sizes, for a build that reads nothing back (CUDA-graph capture).  x / pos / edges /
+ * n_nodes / n_edges come from gnc_build_superpixel_graph called with S_max = S_cap and E_max = E_cap; node_ptr /
+ * edge_ptr from gnc_superpixel_batch_offsets with the same capacities.
+ *   xb float [B * S_cap + 1, 3], pb float [B * S_cap + 1, 2], eb int64 [2, B * E_cap]
+ * Rows [0, node_ptr[B]) and edges [0, edge_ptr[B]) equal gnc_superpixel_batch_compact's output.  The other rows are
+ * zero; the other edges are self-loops of those rows (edge edge_ptr[B] + k loops on row node_ptr[B] + k mod
+ * (B * S_cap + 1 - node_ptr[B])), so no real node receives a padding edge.  `labels` (int32 [B, H, W], may be NULL) is
+ * checked against [0, max_label].  *overflow (int32) is overwritten: 0 when everything fit, else bit 0 = a label out of
+ * range, bit 1 = an image with more than S_cap nodes, bit 2 = more than E_cap edges.  Never writes outside the buffers. */
+int gnc_superpixel_batch_padded(const float* x, const float* pos, const int64_t* edges, const int32_t* n_nodes,
+                                const int32_t* n_edges, const int32_t* labels, int B, int H, int W, int max_label,
+                                int S_cap, int64_t E_cap, const int32_t* node_ptr, const int64_t* edge_ptr, float* xb,
+                                float* pb, int64_t* eb, int32_t* overflow, gnc_stream_t stream);
 
 /* SLIC superpixel labels for B images (the stage the reference delegates to scikit-image,
  * image_to_graph_superpixel.py:31; parity unpinned - see csrc/slic.cu): RGB -> Lab, regular-grid
