@@ -186,12 +186,27 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
 // 12.6 ms instead of 9.2 ms on 16.6 M rows - the N = 64 shape runs well below the N = 128 rate.)
 constexpr uint32_t kInstrDesc = (1u << 4) | (0u << 7) | (0u << 10) | ((128u >> 3) << 17) | ((256u >> 4) << 24);
 
-// (x0, x1), already scaled -> two packed fp16 pairs (low half = x0) with p1 + p2 == x to 22 bits
-__device__ __forceinline__ void split2(float x0, float x1, uint32_t& p1, uint32_t& p2) {
-  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p1) : "f"(x1), "f"(x0));
+// Packed FP32 (sm_100: FFMA2 / FADD2 / FMUL2 act on a 64-bit register pair).  Each lane is the scalar IEEE
+// round-to-nearest operation without flush to zero, so two scalar operations and their packed form give the same
+// bits as long as the order of operations is kept.  The per-element work of loaders and epilogues is written in
+// pairs of adjacent columns with these; ReLU stays scalar (there is no packed max).
+__device__ __forceinline__ float2 pair2(const float* v) { return make_float2(v[0], v[1]); }
+__device__ __forceinline__ void set2(float* v, float2 r) { v[0] = r.x; v[1] = r.y; }
+__device__ __forceinline__ float2 dup2(float s) { return make_float2(s, s); }
+
+// (x0, x1), already scaled -> two packed fp16 pairs (low half = x0) with p1 + p2 == x to 22 bits.  The hi piece is
+// unpacked with two cvt.f32.f16: there is no cheaper exact unpack; the residual x - h is one packed subtraction.
+__device__ __forceinline__ void split2(float2 x, uint32_t& p1, uint32_t& p2) {
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p1) : "f"(x.y), "f"(x.x));
   float h0, h1;
   asm("{.reg .f16 lo, hi; mov.b32 {lo, hi}, %2; cvt.f32.f16 %0, lo; cvt.f32.f16 %1, hi;}" : "=f"(h0), "=f"(h1) : "r"(p1));
-  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p2) : "f"(x1 - h1), "f"(x0 - h0));
+  const float2 r = __fadd2_rn(x, make_float2(-h0, -h1));
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p2) : "f"(r.y), "f"(r.x));
+}
+__device__ __forceinline__ void split2(float x0, float x1, uint32_t& p1, uint32_t& p2) { split2(make_float2(x0, x1), p1, p2); }
+// (x0, x1) x s, s an exact power of two (the operand scalings), then split
+__device__ __forceinline__ void split2_scaled(float x0, float x1, float s, uint32_t& p1, uint32_t& p2) {
+  split2(__fmul2_rn(make_float2(x0, x1), dup2(s)), p1, p2);
 }
 // ReLU that keeps NaN (fmaxf would turn the NaN of an out-of-range fp16 operand into a silent 0)
 __device__ __forceinline__ float relu_nan(float x) {
@@ -334,10 +349,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       const float4 v0 = __ldg(reinterpret_cast<const float4*>(src));
       const float4 v1 = __ldg(reinterpret_cast<const float4*>(src + 4));
       uint32_t p1[4], p2[4];
-      split2(v0.x * kScaleW, v0.y * kScaleW, p1[0], p2[0]);
-      split2(v0.z * kScaleW, v0.w * kScaleW, p1[1], p2[1]);
-      split2(v1.x * kScaleW, v1.y * kScaleW, p1[2], p2[2]);
-      split2(v1.z * kScaleW, v1.w * kScaleW, p1[3], p2[3]);
+      split2_scaled(v0.x, v0.y, kScaleW, p1[0], p2[0]);
+      split2_scaled(v0.z, v0.w, kScaleW, p1[1], p2[1]);
+      split2_scaled(v1.x, v1.y, kScaleW, p1[2], p2[2]);
+      split2_scaled(v1.z, v1.w, kScaleW, p1[3], p2[3]);
       const int kb = c >> 3, cc = c & 7;
       uint8_t* img = sm + kOffW + l * kLayerBytes + kb * kImgBytes + (nloc >> 3) * 1024 + (nloc & 7) * 128 + ((cc ^ (nloc & 7)) << 4);
       *reinterpret_cast<uint4*>(img) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
@@ -406,8 +421,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const float4 x = *reinterpret_cast<const float4*>(buf + (((half * 4 + j) ^ (lane & 7)) << 4));
-          split2(x.x * kScaleA, x.y * kScaleA, p1[2 * j], p2[2 * j]);
-          split2(x.z * kScaleA, x.w * kScaleA, p1[2 * j + 1], p2[2 * j + 1]);
+          split2_scaled(x.x, x.y, kScaleA, p1[2 * j], p2[2 * j]);
+          split2_scaled(x.z, x.w, kScaleA, p1[2 * j + 1], p2[2 * j + 1]);
         }
         tmem_st8(ta + half * 8, p1);
         tmem_st8(ta + 64 + half * 8, p2);
@@ -875,6 +890,49 @@ __device__ __forceinline__ void cp_async_wait_pending(int n) {
   }
 }
 
+// Exact two-pass LayerNorm of a row held by two epilogue warps (this thread's 64 values in x): each pass publishes the
+// half's sum in `mine`, meets the partner warp at named barrier 1 + q and adds the partner's `other`.  The partial
+// sums t0..t3 over columns j = 0, 1, 2, 3 mod 4 run as two packed accumulators (t0, t1), (t2, t3) and are reduced as
+// (t0 + t1) + (t2 + t3).
+__device__ __forceinline__ float row_mean(const float* x, float* mine, const float* other, int q) {
+  float2 ta = dup2(0.f), tb = dup2(0.f);
+#pragma unroll
+  for (int jj = 0; jj < 64; jj += 4) { ta = __fadd2_rn(ta, pair2(x + jj)); tb = __fadd2_rn(tb, pair2(x + jj + 2)); }
+  const float s1 = (ta.x + ta.y) + (tb.x + tb.y);
+  *mine = s1;
+  named_bar_sync(1 + q, 64);
+  return (s1 + *other) * (1.0f / kD);
+}
+// x -= mu in place; returns 1 / sqrt(var + eps)
+__device__ __forceinline__ float row_rstd(float* x, float mu, float* mine, const float* other, int q, float eps) {
+  float2 ta = dup2(0.f), tb = dup2(0.f);
+#pragma unroll
+  for (int jj = 0; jj < 64; jj += 4) {
+    set2(x + jj, __fadd2_rn(pair2(x + jj), dup2(-mu)));
+    set2(x + jj + 2, __fadd2_rn(pair2(x + jj + 2), dup2(-mu)));
+    ta = __ffma2_rn(pair2(x + jj), pair2(x + jj), ta);
+    tb = __ffma2_rn(pair2(x + jj + 2), pair2(x + jj + 2), tb);
+  }
+  const float s2 = (ta.x + ta.y) + (tb.x + tb.y);
+  *mine = s2;
+  named_bar_sync(1 + q, 64);
+  const float var = (s2 + *other) * (1.0f / kD);
+  return 1.0f / sqrtf(var + eps);
+}
+// x = (x rstd) gamma + beta, a multiply then an FMA; x[16 c + i] takes gamma[32 c + i], beta[32 c + i]
+__device__ __forceinline__ void normalise(float* x, float rstd, const float* gamma, const float* beta) {
+#pragma unroll
+  for (int c = 0; c < 4; ++c)
+#pragma unroll
+    for (int j4 = 0; j4 < 4; ++j4) {
+      const float4 g4 = *reinterpret_cast<const float4*>(gamma + 32 * c + 4 * j4);
+      const float4 e4 = *reinterpret_cast<const float4*>(beta + 32 * c + 4 * j4);
+      float* xx = x + 16 * c + 4 * j4;
+      set2(xx, __ffma2_rn(__fmul2_rn(pair2(xx), dup2(rstd)), make_float2(g4.x, g4.y), make_float2(e4.x, e4.y)));
+      set2(xx + 2, __ffma2_rn(__fmul2_rn(pair2(xx + 2), dup2(rstd)), make_float2(g4.z, g4.w), make_float2(e4.z, e4.w)));
+    }
+}
+
 template <int SPEC, bool STASH = false, bool PSUM = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chain2_kernel(const Params p) {
   // STASH (training forward): the hidden ReLU outputs, the LayerNorm input and the row statistics are written out as well
@@ -890,6 +948,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
                 ((kPre && Spec<SPEC>::nl == 2 && Spec<SPEC>::ridx == 1) || (!kPre && Spec<SPEC>::nl == 3 && Spec<SPEC>::ridx == 0)),
                 "two-tile form: addends, LayerNorm, residual; 3 layers, or pre-stage + 2 layers");
   constexpr int nl = Spec<SPEC>::nl;
+  // the pre-stage form has no loader work (the epilogue builds the first operand): its registers go to the epilogue
+  constexpr int kRegsLd = kPre ? 56 : kRegsLoader, kRegsEp = kPre ? 208 : kRegsEpi;
+  static_assert(32 * (4 * kRegsLd + 4 * kRegsMma + kEpiWarps * kRegsEp) <= kThreads * 128, "setmaxnreg budget");
   constexpr bool has_i0 = Spec<SPEC>::i0 != 0, has_g1 = Spec<SPEC>::g1 != 0, has_i1 = Spec<SPEC>::i1 != 0;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
@@ -933,10 +994,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       const float4 v0 = __ldg(reinterpret_cast<const float4*>(src));
       const float4 v1 = __ldg(reinterpret_cast<const float4*>(src + 4));
       uint32_t p1[4], p2[4];
-      split2(v0.x * kScaleW, v0.y * kScaleW, p1[0], p2[0]);
-      split2(v0.z * kScaleW, v0.w * kScaleW, p1[1], p2[1]);
-      split2(v1.x * kScaleW, v1.y * kScaleW, p1[2], p2[2]);
-      split2(v1.z * kScaleW, v1.w * kScaleW, p1[3], p2[3]);
+      split2_scaled(v0.x, v0.y, kScaleW, p1[0], p2[0]);
+      split2_scaled(v0.z, v0.w, kScaleW, p1[1], p2[1]);
+      split2_scaled(v1.x, v1.y, kScaleW, p1[2], p2[2]);
+      split2_scaled(v1.z, v1.w, kScaleW, p1[3], p2[3]);
       const int kb = c >> 3, cc = c & 7;
       uint8_t* img = sm + kOffW + l * kLayerBytes + kb * kImgBytes + (nloc >> 3) * 1024 + (nloc & 7) * 128 + ((cc ^ (nloc & 7)) << 4);
       *reinterpret_cast<uint4*>(img) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
@@ -961,7 +1022,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 
   if (warp < kLoaderWarps) {
     // ======================= loaders =======================
-    reg_dec<kRegsLoader>();
+    reg_dec<kRegsLd>();
     const int q = warp;
     const uint32_t buf0 = base + kOffLd + (uint32_t)(warp * kLoadBufs) * kChunkBytes;
     const int rl = lane >> 3, cj = lane & 7;
@@ -1003,8 +1064,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
         for (int jj = 0; jj < 4; ++jj) {
           const float4 x = *reinterpret_cast<const float4*>(buf + (((half * 4 + jj) ^ (lane & 7)) << 4));
-          split2(x.x * kScaleA, x.y * kScaleA, p1[2 * jj], p2[2 * jj]);
-          split2(x.z * kScaleA, x.w * kScaleA, p1[2 * jj + 1], p2[2 * jj + 1]);
+          split2_scaled(x.x, x.y, kScaleA, p1[2 * jj], p2[2 * jj]);
+          split2_scaled(x.z, x.w, kScaleA, p1[2 * jj + 1], p2[2 * jj + 1]);
         }
         tmem_st8(ta + half * 8, p1);
         tmem_st8(ta + 64 + half * 8, p2);
@@ -1064,7 +1125,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
     __syncwarp();
   } else {
     // ======================= epilogue =======================
-    reg_inc<kRegsEpi>();
+    reg_inc<kRegsEp>();
     const int ew = warp - kEpiWarp0;
     const int q = warp & 3, hf = ew >> 2;
     uint8_t* slots = sm + kOffEp + ew * kEpiSlots * kSlotBytes;
@@ -1141,19 +1202,19 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
       for (int j4 = 0; j4 < 4; ++j4) {
         const float4 b4 = *reinterpret_cast<const float4*>(s_bias + col0 + 4 * j4);
-        float y0 = fmaf(vc[4 * j4], 1.f / kScaleW, b4.x), y1 = fmaf(vc[4 * j4 + 1], 1.f / kScaleW, b4.y);
-        float y2 = fmaf(vc[4 * j4 + 2], 1.f / kScaleW, b4.z), y3 = fmaf(vc[4 * j4 + 3], 1.f / kScaleW, b4.w);
+        float2 ya = __ffma2_rn(pair2(vc + 4 * j4), dup2(1.f / kScaleW), make_float2(b4.x, b4.y));
+        float2 yb = __ffma2_rn(pair2(vc + 4 * j4 + 2), dup2(1.f / kScaleW), make_float2(b4.z, b4.w));
         if (has_ext) {
-          y0 = fmaf(ext[4 * j4], kScaleA, y0); y1 = fmaf(ext[4 * j4 + 1], kScaleA, y1);
-          y2 = fmaf(ext[4 * j4 + 2], kScaleA, y2); y3 = fmaf(ext[4 * j4 + 3], kScaleA, y3);
+          ya = __ffma2_rn(pair2(ext + 4 * j4), dup2(kScaleA), ya);
+          yb = __ffma2_rn(pair2(ext + 4 * j4 + 2), dup2(kScaleA), yb);
         }
-        y0 = relu_nan(y0); y1 = relu_nan(y1); y2 = relu_nan(y2); y3 = relu_nan(y3);
+        ya.x = relu_nan(ya.x); ya.y = relu_nan(ya.y); yb.x = relu_nan(yb.x); yb.y = relu_nan(yb.y);
         if (STASH) {                                // exact: kScaleA is a power of two
-          st[4 * j4] = y0 * (1.f / kScaleA); st[4 * j4 + 1] = y1 * (1.f / kScaleA);
-          st[4 * j4 + 2] = y2 * (1.f / kScaleA); st[4 * j4 + 3] = y3 * (1.f / kScaleA);
+          set2(st + 4 * j4, __fmul2_rn(ya, dup2(1.f / kScaleA)));
+          set2(st + 4 * j4 + 2, __fmul2_rn(yb, dup2(1.f / kScaleA)));
         }
-        split2(y0, y1, p1[2 * j4], p2[2 * j4]);
-        split2(y2, y3, p1[2 * j4 + 1], p2[2 * j4 + 1]);
+        split2(ya, p1[2 * j4], p2[2 * j4]);
+        split2(yb, p1[2 * j4 + 1], p2[2 * j4 + 1]);
       }
       if (STASH && strow) { stg256(strow + col0, st); stg256(strow + col0 + 8, st + 8); }
       const uint32_t ta = lane_addr + (uint32_t)S * 256 + 128 + (uint32_t)(16 * c + 8 * hf);
@@ -1216,7 +1277,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
             float e1[16];
             read_slot(sp + kSlotBytes, e1);
 #pragma unroll
-            for (int jj = 0; jj < 16; ++jj) ext[jj] += e1[jj];
+            for (int jj = 0; jj < 16; jj += 2) set2(ext + jj, __fadd2_rn(pair2(ext + jj), pair2(e1 + jj)));
           }
           __syncwarp();
           // next issue of the stream: two addend steps stay in flight; after a tile's last two steps the
@@ -1238,7 +1299,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
             for (int j4 = 0; j4 < 4; ++j4) {
               const float4 r4 = __ldg(reinterpret_cast<const float4*>(trow + 32 * c + 4 * j4));
-              ext[4 * j4] += r4.x; ext[4 * j4 + 1] += r4.y; ext[4 * j4 + 2] += r4.z; ext[4 * j4 + 3] += r4.w;
+              set2(ext + 4 * j4, __fadd2_rn(pair2(ext + 4 * j4), make_float2(r4.x, r4.y)));
+              set2(ext + 4 * j4 + 2, __fadd2_rn(pair2(ext + 4 * j4 + 2), make_float2(r4.z, r4.w)));
             }
             mbar_wait(a_empty(S, c), (uint32_t)((g & 1) ^ 1));      // the slot's previous tile has read chunk c
             tc_fence_after();
@@ -1289,8 +1351,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
           for (int j4 = 0; j4 < 4; ++j4) {
             const float4 b4 = *reinterpret_cast<const float4*>(s_bias + 32 * c + 16 * hf + 4 * j4);
             float* xx = x + 16 * c + 4 * j4;
-            xx[0] = fmaf(xx[0], kUnscaleD, b4.x); xx[1] = fmaf(xx[1], kUnscaleD, b4.y);
-            xx[2] = fmaf(xx[2], kUnscaleD, b4.z); xx[3] = fmaf(xx[3], kUnscaleD, b4.w);
+            set2(xx, __ffma2_rn(pair2(xx), dup2(kUnscaleD), make_float2(b4.x, b4.y)));
+            set2(xx + 2, __ffma2_rn(pair2(xx + 2), dup2(kUnscaleD), make_float2(b4.z, b4.w)));
           }
         const bool st_row = STASH && row0 + lane < p.M;
         if (STASH && st_row) {                                      // the LayerNorm input, as the backward reads it
@@ -1301,37 +1363,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
         float* xa = xchg + (ew * 32 + lane);
         float* xb = xchg + (kEpiWarps * 32) + (ew * 32 + lane);
         const int partner = (ew ^ 4) * 32 + lane;
-        float t0 = 0.f, t1 = 0.f, t2 = 0.f, t3 = 0.f;
-#pragma unroll
-        for (int jj = 0; jj < 64; jj += 4) { t0 += x[jj]; t1 += x[jj + 1]; t2 += x[jj + 2]; t3 += x[jj + 3]; }
-        const float s1 = (t0 + t1) + (t2 + t3);
-        *xa = s1;
-        named_bar_sync(1 + q, 64);
-        const float mu = (s1 + xchg[partner]) * (1.0f / kD);
-        t0 = t1 = t2 = t3 = 0.f;
-#pragma unroll
-        for (int jj = 0; jj < 64; jj += 4) {
-          x[jj] -= mu; x[jj + 1] -= mu; x[jj + 2] -= mu; x[jj + 3] -= mu;
-          t0 = fmaf(x[jj], x[jj], t0); t1 = fmaf(x[jj + 1], x[jj + 1], t1);
-          t2 = fmaf(x[jj + 2], x[jj + 2], t2); t3 = fmaf(x[jj + 3], x[jj + 3], t3);
-        }
-        const float s2 = (t0 + t1) + (t2 + t3);
-        *xb = s2;
-        named_bar_sync(1 + q, 64);
-        const float var = (s2 + xchg[kEpiWarps * 32 + partner]) * (1.0f / kD);
-        const float rstd = 1.0f / sqrtf(var + p.eps);
+        const float mu = row_mean(x, xa, xchg + partner, q);
+        const float rstd = row_rstd(x, mu, xb, xchg + kEpiWarps * 32 + partner, q, p.eps);
         if (STASH && st_row && hf == 0) { p.st_mean[row0 + lane] = mu; p.st_rstd[row0 + lane] = rstd; }
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-#pragma unroll
-          for (int j4 = 0; j4 < 4; ++j4) {
-            const int col = 32 * c + 16 * hf + 4 * j4;
-            const float4 g4 = *reinterpret_cast<const float4*>(s_const + 3 * kD + col);
-            const float4 e4 = *reinterpret_cast<const float4*>(s_const + 4 * kD + col);
-            float* xx = x + 16 * c + 4 * j4;
-            xx[0] = fmaf(xx[0] * rstd, g4.x, e4.x); xx[1] = fmaf(xx[1] * rstd, g4.y, e4.y);
-            xx[2] = fmaf(xx[2] * rstd, g4.z, e4.z); xx[3] = fmaf(xx[3] * rstd, g4.w, e4.w);
-          }
+        normalise(x, rstd, s_const + 3 * kD + 16 * hf, s_const + 4 * kD + 16 * hf);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           uint8_t* slot = slots + c * kSlotBytes;
@@ -1339,7 +1374,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
             for (int j4 = 0; j4 < 4; ++j4) {
               const float4 r4 = __ldg(reinterpret_cast<const float4*>(rrow + 32 * c + 4 * j4));
-              x[16 * c + 4 * j4] += r4.x; x[16 * c + 4 * j4 + 1] += r4.y; x[16 * c + 4 * j4 + 2] += r4.z; x[16 * c + 4 * j4 + 3] += r4.w;
+              float* xx = x + 16 * c + 4 * j4;
+              set2(xx, __fadd2_rn(pair2(xx), make_float2(r4.x, r4.y)));
+              set2(xx + 2, __fadd2_rn(pair2(xx + 2), make_float2(r4.z, r4.w)));
             }
           } else {
             wait_next();                                            // residual step c of this tile
@@ -1347,7 +1384,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
             float rsd[16];
             read_slot(slot, rsd);
 #pragma unroll
-            for (int jj = 0; jj < 16; ++jj) x[16 * c + jj] += rsd[jj];
+            for (int jj = 0; jj < 16; jj += 2) set2(x + 16 * c + jj, __fadd2_rn(pair2(x + 16 * c + jj), pair2(rsd + jj)));
             __syncwarp();
           }
           if (pad_row) {
@@ -1365,8 +1402,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
               const int nr = rl + 8 * k;
               const float4 a = *reinterpret_cast<const float4*>(slot + slot_off(2 * nr, cc));
               const float4 b = *reinterpret_cast<const float4*>(slot + slot_off(2 * nr + 1, cc));
-              const float4 o = make_float4(__fadd_rn(__fadd_rn(0.f, a.x), b.x), __fadd_rn(__fadd_rn(0.f, a.y), b.y),
-                                           __fadd_rn(__fadd_rn(0.f, a.z), b.z), __fadd_rn(__fadd_rn(0.f, a.w), b.w));
+              const float2 o01 = __fadd2_rn(__fadd2_rn(dup2(0.f), make_float2(a.x, a.y)), make_float2(b.x, b.y));
+              const float2 o23 = __fadd2_rn(__fadd2_rn(dup2(0.f), make_float2(a.z, a.w)), make_float2(b.z, b.w));
+              const float4 o = make_float4(o01.x, o01.y, o23.x, o23.y);
               if (tile_full || row0 + 2 * nr < p.M)
                 stg_hint(reinterpret_cast<float4*>(p.Y + ((row0 >> 1) + nr) * p.ldy + 32 * c + 16 * hf + 4 * cc), o, pol_drop);
             }
@@ -1417,7 +1455,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
   // PAIR (an AGG form): A is the paired destination slot table (gnc_grid_pair_slots) and row m's edge rows are the adjacent
   // rows 2m, 2m + 1 (a zero row where an edge is missing) - the same two sources, with addresses instead of index lookups.
   static_assert(!PAIR || AGG, "PAIR is a form of AGG");
-  constexpr int kRegsLd = AGG ? 88 : kRegsLoader, kRegsEp = AGG ? 192 : kRegsEpi;
+  // loaders that form their operand (AGG, PAIR, SYN) take registers from the epilogue: the smallest splits without spills
+  constexpr int kRegsLd = PAIR ? 96 : (AGG || SYN) ? 88 : kRegsLoader, kRegsEp = PAIR ? 184 : (AGG || SYN) ? 192 : kRegsEpi;
   static_assert(32 * (4 * kRegsLd + 4 * kRegsMma + kEpiWarps * kRegsEp) <= kThreads * 128, "setmaxnreg budget");
   constexpr int kImgs = NL + (K2 ? 1 : 0);
   static_assert(kImgs <= 4 && NL >= 2, "at most four weight images");
@@ -1473,22 +1512,23 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
       const float4 v0 = __ldg(reinterpret_cast<const float4*>(src));
       const float4 v1 = __ldg(reinterpret_cast<const float4*>(src + 4));
       uint32_t p1[4], p2[4];
-      split2(v0.x * kScaleW, v0.y * kScaleW, p1[0], p2[0]);
-      split2(v0.z * kScaleW, v0.w * kScaleW, p1[1], p2[1]);
-      split2(v1.x * kScaleW, v1.y * kScaleW, p1[2], p2[2]);
-      split2(v1.z * kScaleW, v1.w * kScaleW, p1[3], p2[3]);
+      split2_scaled(v0.x, v0.y, kScaleW, p1[0], p2[0]);
+      split2_scaled(v0.z, v0.w, kScaleW, p1[1], p2[1]);
+      split2_scaled(v1.x, v1.y, kScaleW, p1[2], p2[2]);
+      split2_scaled(v1.z, v1.w, kScaleW, p1[3], p2[3]);
       const int kb = c >> 3, cc = c & 7;
       uint8_t* img = sm + im * kLayerBytes + kb * kImgBytes + (nloc >> 3) * 1024 + (nloc & 7) * 128 + ((cc ^ (nloc & 7)) << 4);
       *reinterpret_cast<uint4*>(img) = make_uint4(p1[0], p1[1], p1[2], p1[3]);
       *reinterpret_cast<uint4*>(img + 2 * kImgBytes) = make_uint4(p2[0], p2[1], p2[2], p2[3]);
     }
   }
-  // SYN: the narrow layer's weights live where the (unused) loader ring would be: per output column 8 weights
-  // (zero-padded) + the bias, all x kScaleA (the loader emits the scaled operand; ReLU commutes with the scaling)
+  // SYN: the narrow layer's weights live where the (unused) loader ring would be, all x kScaleA (the loader emits the
+  // scaled operand; ReLU commutes with the scaling).  Per pair of output columns (2k, 2k + 1) 20 floats: the 8 weights
+  // (zero-padded) interleaved column by column, then the two biases and two zeros - operand pairs of packed FMAs.
   float* s_syn = reinterpret_cast<float*>(sm + kOffLd2);
   if (SYN) {
-    for (int i = threadIdx.x; i < kD * 12; i += kThreads) {
-      const int col = i / 12, j = i - col * 12;
+    for (int i = threadIdx.x; i < kD * 10; i += kThreads) {
+      const int k = i / 20, r = i - k * 20, col = 2 * k + (r & 1), j = r >> 1;
       float v = 0.f;
       if (j < p.syn_k) v = __ldg(p.syn_W + (long long)col * p.ld_syn_W + j) * kScaleA;
       else if (j == 8) v = p.syn_b ? __ldg(p.syn_b + col) * kScaleA : 0.f;
@@ -1657,33 +1697,33 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
         uint32_t p1[8], p2[8];
         if (SYN) {
 #pragma unroll
-          for (int jj = 0; jj < 8; ++jj) {
-            float y[2];
+          for (int jj = 0; jj < 8; ++jj) {           // columns c * 32 + half * 16 + 2 jj, + 1 (one packed lane each)
+            const float* w = s_syn + (c * 16 + half * 8 + jj) * 20;
+            float2 acc = *reinterpret_cast<const float2*>(w + 16);
 #pragma unroll
-            for (int e = 0; e < 2; ++e) {
-              const float* w = s_syn + (c * 32 + half * 16 + 2 * jj + e) * 12;
-              const float4 w0 = *reinterpret_cast<const float4*>(w), w1 = *reinterpret_cast<const float4*>(w + 4);
-              float acc = w[8];
-              acc = fmaf(xin[0], w0.x, acc); acc = fmaf(xin[1], w0.y, acc); acc = fmaf(xin[2], w0.z, acc); acc = fmaf(xin[3], w0.w, acc);
-              acc = fmaf(xin[4], w1.x, acc); acc = fmaf(xin[5], w1.y, acc); acc = fmaf(xin[6], w1.z, acc); acc = fmaf(xin[7], w1.w, acc);
-              y[e] = relu_nan(acc);
+            for (int t = 0; t < 8; t += 2) {
+              const float4 wt = *reinterpret_cast<const float4*>(w + 2 * t);     // weights t, t + 1 of both columns
+              acc = __ffma2_rn(dup2(xin[t]), make_float2(wt.x, wt.y), acc);
+              acc = __ffma2_rn(dup2(xin[t + 1]), make_float2(wt.z, wt.w), acc);
             }
-            split2(y[0], y[1], p1[jj], p2[jj]);
+            split2(relu_nan(acc.x), relu_nan(acc.y), p1[jj], p2[jj]);
           }
         } else {
 #pragma unroll
           for (int jj = 0; jj < 4; ++jj) {
-            float4 x = *reinterpret_cast<const float4*>(buf + (((half * 4 + jj) ^ (lane & 7)) << 4));
+            const float4 x = *reinterpret_cast<const float4*>(buf + (((half * 4 + jj) ^ (lane & 7)) << 4));
+            float2 xa = make_float2(x.x, x.y), xb = make_float2(x.z, x.w);
             if (PAIR && op == 0) {                    // (0 + a) + b, a = row 2m (horizontal), b = row 2m + 1 (vertical)
               const float* y = x2 + 16 * half + 4 * jj;
-              x.x = __fadd_rn(__fadd_rn(0.f, x.x), y[0]); x.y = __fadd_rn(__fadd_rn(0.f, x.y), y[1]);
-              x.z = __fadd_rn(__fadd_rn(0.f, x.z), y[2]); x.w = __fadd_rn(__fadd_rn(0.f, x.w), y[3]);
+              xa = __fadd2_rn(__fadd2_rn(dup2(0.f), xa), pair2(y));
+              xb = __fadd2_rn(__fadd2_rn(dup2(0.f), xb), pair2(y + 2));
             } else if (AGG && op == 0) {              // (0 + a) + b: the ordered sum of the row's edges
               const float* y = x2 + 16 * half + 4 * jj;
-              x.x += y[0]; x.y += y[1]; x.z += y[2]; x.w += y[3];
+              xa = __fadd2_rn(xa, pair2(y));
+              xb = __fadd2_rn(xb, pair2(y + 2));
             }
-            split2(x.x * kScaleA, x.y * kScaleA, p1[2 * jj], p2[2 * jj]);
-            split2(x.z * kScaleA, x.w * kScaleA, p1[2 * jj + 1], p2[2 * jj + 1]);
+            split2(__fmul2_rn(xa, dup2(kScaleA)), p1[2 * jj], p2[2 * jj]);
+            split2(__fmul2_rn(xb, dup2(kScaleA)), p1[2 * jj + 1], p2[2 * jj + 1]);
           }
         }
         tmem_st8(ta + half * 8, p1);
@@ -1816,10 +1856,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
 #pragma unroll
       for (int j4 = 0; j4 < 4; ++j4) {
         const float4 b4 = *reinterpret_cast<const float4*>(s_bias + col0 + 4 * j4);
-        const float y0 = fmaf(vc[4 * j4], 1.f / kScaleW, b4.x), y1 = fmaf(vc[4 * j4 + 1], 1.f / kScaleW, b4.y);
-        const float y2 = fmaf(vc[4 * j4 + 2], 1.f / kScaleW, b4.z), y3 = fmaf(vc[4 * j4 + 3], 1.f / kScaleW, b4.w);
-        split2(relu_nan(y0), relu_nan(y1), p1[2 * j4], p2[2 * j4]);
-        split2(relu_nan(y2), relu_nan(y3), p1[2 * j4 + 1], p2[2 * j4 + 1]);
+        const float2 ya = __ffma2_rn(pair2(vc + 4 * j4), dup2(1.f / kScaleW), make_float2(b4.x, b4.y));
+        const float2 yb = __ffma2_rn(pair2(vc + 4 * j4 + 2), dup2(1.f / kScaleW), make_float2(b4.z, b4.w));
+        split2(relu_nan(ya.x), relu_nan(ya.y), p1[2 * j4], p2[2 * j4]);
+        split2(relu_nan(yb.x), relu_nan(yb.y), p1[2 * j4 + 1], p2[2 * j4 + 1]);
       }
       const uint32_t ta = lane_addr + (uint32_t)S * 256 + 128 + (uint32_t)(16 * c + 8 * hf);
       tmem_st8(ta, p1);
@@ -1873,8 +1913,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
           for (int j4 = 0; j4 < 4; ++j4) {
             const float4 b4 = *reinterpret_cast<const float4*>(s_bias + 32 * c + 16 * hf + 4 * j4);
             float* xx = x + 16 * c + 4 * j4;
-            xx[0] = fmaf(xx[0], kUnscaleD, b4.x); xx[1] = fmaf(xx[1], kUnscaleD, b4.y);
-            xx[2] = fmaf(xx[2], kUnscaleD, b4.z); xx[3] = fmaf(xx[3], kUnscaleD, b4.w);
+            set2(xx, __ffma2_rn(pair2(xx), dup2(kUnscaleD), make_float2(b4.x, b4.y)));
+            set2(xx + 2, __ffma2_rn(pair2(xx + 2), dup2(kUnscaleD), make_float2(b4.z, b4.w)));
           }
         float* xa = xchg + (ew * 32 + lane);
         float* xb = xchg + (kEpiWarps * 32) + (ew * 32 + lane);
@@ -1897,36 +1937,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
           continue;
         }
         if (p.gamma) {
-          float t0 = 0.f, t1 = 0.f, t2 = 0.f, t3 = 0.f;
-#pragma unroll
-          for (int jj = 0; jj < 64; jj += 4) { t0 += x[jj]; t1 += x[jj + 1]; t2 += x[jj + 2]; t3 += x[jj + 3]; }
-          const float s1 = (t0 + t1) + (t2 + t3);
-          *xa = s1;
-          named_bar_sync(1 + q, 64);
-          const float mu = (s1 + xchg[partner]) * (1.0f / kD);
-          t0 = t1 = t2 = t3 = 0.f;
-#pragma unroll
-          for (int jj = 0; jj < 64; jj += 4) {
-            x[jj] -= mu; x[jj + 1] -= mu; x[jj + 2] -= mu; x[jj + 3] -= mu;
-            t0 = fmaf(x[jj], x[jj], t0); t1 = fmaf(x[jj + 1], x[jj + 1], t1);
-            t2 = fmaf(x[jj + 2], x[jj + 2], t2); t3 = fmaf(x[jj + 3], x[jj + 3], t3);
-          }
-          const float s2 = (t0 + t1) + (t2 + t3);
-          *xb = s2;
-          named_bar_sync(1 + q, 64);
-          const float var = (s2 + xchg[kEpiWarps * 32 + partner]) * (1.0f / kD);
-          const float rstd = 1.0f / sqrtf(var + p.eps);
-#pragma unroll
-          for (int c = 0; c < 4; ++c)
-#pragma unroll
-            for (int j4 = 0; j4 < 4; ++j4) {
-              const int col = 32 * c + 16 * hf + 4 * j4;
-              const float4 g4 = *reinterpret_cast<const float4*>(s_const + 3 * kD + col);
-              const float4 e4 = *reinterpret_cast<const float4*>(s_const + 4 * kD + col);
-              float* xx = x + 16 * c + 4 * j4;
-              xx[0] = fmaf(xx[0] * rstd, g4.x, e4.x); xx[1] = fmaf(xx[1] * rstd, g4.y, e4.y);
-              xx[2] = fmaf(xx[2] * rstd, g4.z, e4.z); xx[3] = fmaf(xx[3] * rstd, g4.w, e4.w);
-            }
+          const float mu = row_mean(x, xa, xchg + partner, q);
+          const float rstd = row_rstd(x, mu, xb, xchg + kEpiWarps * 32 + partner, q, p.eps);
+          normalise(x, rstd, s_const + 3 * kD + 16 * hf, s_const + 4 * kD + 16 * hf);
         }
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
@@ -1940,7 +1953,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1) tc_chai
             float rsd[16];
             read_slot(slot, rsd);
 #pragma unroll
-            for (int jj = 0; jj < 16; ++jj) x[16 * c + jj] += rsd[jj];
+            for (int jj = 0; jj < 16; jj += 2) set2(x + 16 * c + jj, __fadd2_rn(pair2(x + 16 * c + jj), pair2(rsd + jj)));
             __syncwarp();
           }
 #pragma unroll
