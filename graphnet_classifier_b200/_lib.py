@@ -73,6 +73,21 @@ class GncJpegImage(Structure):
                 ("quant", (c_uint16 * 64) * 4), ("huff", GncJpegHuff * 8)]
 
 
+class GncJpegScan(Structure):
+    """struct gnc_jpeg_scan (include/gnc.h)."""
+    _fields_ = [("image", c_int32), ("ncomp", c_int32), ("comp", c_int32 * 3), ("dc_tab", c_int32 * 3), ("ac_tab", c_int32),
+                ("Ss", c_int32), ("Se", c_int32), ("Ah", c_int32), ("Al", c_int32), ("restart_interval", c_int32),
+                ("offset", c_int64), ("bytes", c_int64)]
+
+
+class GncJpegChain(Structure):
+    """struct gnc_jpeg_chain (include/gnc.h)."""
+    _fields_ = [("first_scan", c_int32), ("n_scans", c_int32), ("bytes", c_int64)]
+
+
+GNC_JPEG_MAX_SCANS, GNC_JPEG_MAX_TABLES = 64, 32
+
+
 class GncError(RuntimeError):
     pass
 
@@ -162,6 +177,10 @@ SIGNATURES = {
     "gnc_jpeg_scratch_bytes": (c_int64, [c_int64, c_int]),
     "gnc_jpeg_decode_rgb_u8": (c_int, [_P, _P, c_int, c_int64, c_int64, _P, _P, _P, _P, _P]),
     "gnc_debug_jpeg_sequential": (c_int, [c_int]),
+    "gnc_jpeg_pack_progressive": (c_int, [_P, _P, c_int, c_int, _P, c_int64, _P, _P, _P, c_int64, _P, c_int64, _P, c_int64,
+                                          _P]),
+    "gnc_jpeg_decode_progressive_rgb_u8": (c_int, [_P, _P, c_int, _P, _P, c_int, _P, c_int64, c_int64, _P, _P, _P, _P]),
+    "gnc_debug_jpeg_chains_per_warp": (c_int, [c_int]),
     "gnc_tc_bwd_layer_parts": (c_int32, [c_int64]),
     "gnc_tc_bwd_reduce_batch_f32": (c_int, [POINTER(GncBwdReduceItem), c_int32, _P]),
 }

@@ -4,7 +4,7 @@ utils/image_to_graph/image_to_graph_optimized.py:65-70, utils/inference.py:47). 
 
 * baseline JPEG files are decoded ON THE DEVICE (``utils/jpeg.py``, csrc/jpeg.cu: libjpeg's integer algorithm restated,
   bit for bit Pillow's pixels): the pool's threads only read the files and parse their markers, and only the compressed
-  bytes cross PCIe;
+  bytes cross PCIe; with ``device_jpeg="progressive"`` progressive JPEG files are decoded on the device too;
 * everything else (PNG, progressive / CMYK JPEG, ...; or all files with ``device_jpeg=False``): the decode
   (``Image.open`` + ``convert('RGB')``: libjpeg inside Pillow) runs on a pool of host PROCESSES (Pillow's
   Python-level file handling holds the GIL for about half of a small file's decode time: 8 threads give 2 x one
@@ -82,7 +82,8 @@ class DecodePool:
         self._shared = [None, None]
         # baseline JPEG files: Huffman + IDCT + colour on the GPU ("auto" = yes): 63 k files/s per GPU against ~1.3 k per
         # host core, only the compressed bytes cross PCIe, and the pixels are Pillow's bit for bit.  Files the device
-        # decoder does not cover take the host path below either way.
+        # decoder does not cover take the host path below either way.  "progressive": progressive files on the device too.
+        self.progressive_jpeg = device_jpeg == "progressive"
         if device_jpeg == "auto":
             device_jpeg = True
         self.device_jpeg = bool(device_jpeg)
@@ -177,7 +178,8 @@ class DecodePool:
         r = int(resize_value)
         pairs, host = chunk["jpeg"], chunk["host"]
         datas = [d if i not in host else b"" for i, (d, _) in enumerate(pairs)]
-        imgs = gjpeg.decode_batch(datas, self.device, staging=self._jpeg_staging[chunk["slot"]])
+        imgs = gjpeg.decode_batch(datas, self.device, staging=self._jpeg_staging[chunk["slot"]],
+                                  progressive=self.progressive_jpeg)
         late = [i for i, t in enumerate(imgs) if t is None and i not in host]     # JPEGs outside the device decoder's scope
         if late:
             host = dict(host)

@@ -196,6 +196,54 @@ int gnc_jpeg_decode_rgb_u8(const uint8_t* stream, const gnc_jpeg_image_t* infos,
 /* Debug aid: 1 = the entropy stage always runs its sequential form (one thread per image); same coefficients. */
 int gnc_debug_jpeg_sequential(int on);
 
+/* Progressive JPEG files (SOF2, 8-bit Huffman, greyscale or YCbCr 4:4:4 / 4:2:2 / 4:2:0), bit for bit what Pillow's
+ * libjpeg produces (csrc/jpeg.cu).  A progressive file codes its coefficients in several scans; every scan writes one
+ * band Ss..Se of one component (AC) or coefficient 0 of one or more components (DC), at bit position Al, refining
+ * (Ah != 0) or first (Ah == 0).  Two scans are linked when they write a common coefficient of a common component; a
+ * CHAIN is a connected group of linked scans in file order.  Chains write disjoint coefficients and decode concurrently.
+ * gnc_jpeg_pack_progressive (HOST): the batch form of gnc_jpeg_pack for progressive files.  Per file that is in:
+ *   frames_out[j]  geometry, MCU counts, n_blocks, plane_bytes, block / coef / plane / pixel offsets and the
+ *                  quantisation tables latched at each component's first scan (qtab[c] = c) - what jpeg_idct_kernel and
+ *                  jpeg_color_kernel read; its huff[] and scan fields are unused;
+ *   its scans      gnc_jpeg_scan_t, entropy segments as offsets into stream_out, tables as indices into tables_out;
+ *   its chains     gnc_jpeg_chain_t, ordered longest first (entropy bytes) across the batch, each chain's scans
+ *                  contiguous in scans_out in file order.
+ *   Left out (index_out lists the files that are in): every file libjpeg would not decode by the plain path - other
+ *   frame types and layouts, progressions jdphuff.c rejects or warns about, and files that end with a DC never coded or
+ *   an AC coefficient 1..9 of some component not fully refined (libjpeg then smooths across blocks) - and files with a
+ *   scan running past the file, no EOI, a DNL, or more than GNC_JPEG_MAX_SCANS scans / GNC_JPEG_MAX_TABLES tables.
+ *   Capacities: scans n * GNC_JPEG_MAX_SCANS, chains the same, tables n * GNC_JPEG_MAX_TABLES always suffice.
+ *   totals[8] = { files in, stream bytes, total blocks, plane bytes, pixels, scans, chains, tables }.
+ * gnc_jpeg_decode_progressive_rgb_u8 (DEVICE): zeroes coef, decodes every chain (one lane per chain, one chain per warp
+ *   by default; scans in file order, jdphuff.c's DC / AC first / refine procedures), then runs the
+ *   baseline IDCT and colour stages on `frames`.  Sizes and buffers as gnc_jpeg_decode_rgb_u8. */
+#define GNC_JPEG_MAX_SCANS 64
+#define GNC_JPEG_MAX_TABLES 32
+typedef struct gnc_jpeg_scan {
+  int32_t image;          /* index into frames */
+  int32_t ncomp;          /* components in the scan; > 1 only for DC scans, which are then interleaved */
+  int32_t comp[3];        /* frame component indices, in frame order */
+  int32_t dc_tab[3];      /* DC first scans: index into tables, per scan component */
+  int32_t ac_tab;         /* AC scans: index into tables */
+  int32_t Ss, Se, Ah, Al;
+  int32_t restart_interval;
+  int64_t offset, bytes;  /* entropy-coded segment in the stream */
+} gnc_jpeg_scan_t;
+typedef struct gnc_jpeg_chain {
+  int32_t first_scan, n_scans;
+  int64_t bytes;          /* entropy bytes of its scans */
+} gnc_jpeg_chain_t;
+int gnc_jpeg_pack_progressive(const uint8_t* const* datas, const int64_t* sizes, int n, int threads, uint8_t* stream_out,
+                              int64_t stream_capacity, gnc_jpeg_image_t* frames_out, int32_t* index_out,
+                              gnc_jpeg_scan_t* scans_out, int64_t scan_capacity, gnc_jpeg_chain_t* chains_out,
+                              int64_t chain_capacity, gnc_jpeg_huff_t* tables_out, int64_t table_capacity, int64_t* totals);
+int gnc_jpeg_decode_progressive_rgb_u8(const uint8_t* stream, const gnc_jpeg_image_t* frames, int B,
+                                       const gnc_jpeg_scan_t* scans, const gnc_jpeg_chain_t* chains, int n_chains,
+                                       const gnc_jpeg_huff_t* tables, int64_t total_blocks, int64_t total_pixels,
+                                       int16_t* coef, uint8_t* planes, uint8_t* out, gnc_stream_t stream_);
+/* Debug aid: chains per warp of the progressive entropy kernel (1..32; anything else = the default, 1).  Same result. */
+int gnc_debug_jpeg_chains_per_warp(int n);
+
 /* Input staging: the resize the reference applies to every image before building its graph,
  *   Image.open(path).convert('RGB').resize((r, r))     utils/image_to_graph/image_to_graph_optimized.py:65-70,
  *                                                      image_to_graph_patch.py / _superpixel.py likewise

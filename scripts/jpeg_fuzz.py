@@ -1,7 +1,12 @@
 #!/usr/bin/env python
 """Randomised check of the device JPEG decoder against Pillow: N files of random size (1 .. 700), content (smooth, noisy,
 flat, text-like edges), quality (5 .. 100), chroma layout, Huffman-table optimisation and restart interval, decoded in
-batches of 64 (images of every kind side by side).  Every pixel must match."""
+batches of 64 (images of every kind side by side).  Every pixel must match.
+
+    jpeg_fuzz.py [N] [SEED] [--progressive]
+
+--progressive: about half the files are saved progressive (Pillow's script, also with restart intervals) and the batches
+go through decode_batch(..., progressive=True); every file must come back decoded."""
 import io, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -9,8 +14,13 @@ from PIL import Image
 from graphnet_classifier_b200 import build
 build.build()
 from graphnet_classifier_b200.utils import jpeg as gjpeg
-N = int(sys.argv[1]) if len(sys.argv) > 1 else 256
-rng = np.random.default_rng(int(sys.argv[2]) if len(sys.argv) > 2 else 0)
+PROGRESSIVE = "--progressive" in sys.argv
+args = [a for a in sys.argv[1:] if not a.startswith("--")]
+N = int(args[0]) if args else 256
+if PROGRESSIVE:
+    from PIL import ImageFile
+    ImageFile.MAXBLOCK = 1 << 25        # Pillow's progressive encoder buffer is W * H bytes: noisy 4:4:4 content overflows it
+rng = np.random.default_rng(int(args[1]) if len(args) > 1 else 0)
 
 
 def image(h, w):
@@ -33,6 +43,10 @@ for i in range(N):
     kw = dict(quality=int(rng.integers(5, 101)), subsampling=int(rng.integers(0, 3)), optimize=bool(rng.integers(0, 2)))
     if rng.random() < 0.15:
         kw["restart_marker_blocks"] = int(rng.integers(1, 20))
+    if PROGRESSIVE and rng.random() < 0.5:
+        kw["progressive"] = True
+        if rng.random() < 0.1:
+            kw["restart_marker_rows"] = int(rng.integers(1, 4))
     im = Image.fromarray(image(h, w))
     if rng.random() < 0.15:
         im = im.convert("L"); kw.pop("subsampling")
@@ -40,12 +54,12 @@ for i in range(N):
     try:
         im.save(buf, format="JPEG", **kw)
     except OSError:                               # Pillow's encoder rejects a few parameter combinations
-        kw.pop("restart_marker_blocks", None); kw["optimize"] = False
+        kw.pop("restart_marker_blocks", None); kw.pop("restart_marker_rows", None); kw["optimize"] = False
         buf = io.BytesIO(); im.save(buf, format="JPEG", **kw)
     datas.append(buf.getvalue()); kws.append((h, w, kw))
 bad = big = 0
 for lo in range(0, N, 64):
-    out = gjpeg.decode_batch(datas[lo:lo + 64])
+    out = gjpeg.decode_batch(datas[lo:lo + 64], progressive=PROGRESSIVE)
     torch.cuda.synchronize()
     for d, t, kw in zip(datas[lo:lo + 64], out, kws[lo:lo + 64]):
         ref = np.asarray(Image.open(io.BytesIO(d)).convert("RGB"))
@@ -53,5 +67,6 @@ for lo in range(0, N, 64):
         if t is None or t.shape != ref.shape or not np.array_equal(t.cpu().numpy(), ref):
             bad += 1
             print("MISMATCH", kw, None if t is None else int(np.abs(t.cpu().numpy().astype(int) - ref).max()))
-print(f"{N} files ({big} large enough for the parallel entropy decoder): {bad} mismatches")
+n_prog = sum(bool(kw.get("progressive")) for _, _, kw in kws)
+print(f"{N} files ({n_prog} progressive, {big} large enough for the parallel entropy decoder): {bad} mismatches")
 sys.exit(1 if bad else 0)
