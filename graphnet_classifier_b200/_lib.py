@@ -88,6 +88,12 @@ class GncJpegChain(Structure):
 GNC_JPEG_MAX_SCANS, GNC_JPEG_MAX_TABLES = 64, 32
 
 
+class GncResizeImage(Structure):
+    """struct gnc_resize_image (include/gnc.h)."""
+    _fields_ = [("src", c_void_p), ("pitch", c_int64), ("tmp_row", c_int64), ("tab_x", c_int64), ("tab_y", c_int64),
+                ("height", c_int32), ("width", c_int32), ("ksize_x", c_int32), ("ksize_y", c_int32)]
+
+
 class GncError(RuntimeError):
     pass
 
@@ -112,6 +118,7 @@ SIGNATURES = {
     "gnc_resize_bicubic_coeffs": (c_int, [c_int, c_int, _P, _P]),
     "gnc_resize_bicubic_u8": (c_int, [_P, c_int64, c_int, c_int, c_int64, c_int64, c_int, c_int, _P, _P, c_int, _P, _P, c_int,
                                       _P, _P, _P]),
+    "gnc_resize_bicubic_ragged_u8": (c_int, [_P, c_int64, c_int, c_int, c_int64, c_int, _P, _P, _P, _P]),
     "gnc_csr_workspace": (c_int64, [c_int64]),
     "gnc_csr_build": (c_int, [_P, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, _P]),
     "gnc_agg_csr_sum_f32": (c_int, [_P, _P, _P, c_int64, c_int64, c_int, _P, c_int64, c_int, _P]),

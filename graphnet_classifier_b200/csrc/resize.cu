@@ -249,24 +249,8 @@ static int launch_h_long(const uint8_t* src, int64_t B, int H, int W, int64_t pi
   return check_launch("resize_h_long_kernel");
 }
 
-// src: [B] images of H rows x row_bytes (pitch / image_stride in bytes); dst: [B, OH, row_bytes] contiguous.
-// One thread per 32-bit word of the output (flattened over rows, so narrow rows still fill the CTAs).
-__global__ void __launch_bounds__(kThreads) resize_v_kernel(const uint8_t* __restrict__ src, int row_bytes, long long pitch,
-                                                             long long image_stride, int OH, long long n_rows,
-                                                             const int32_t* __restrict__ bounds, const int32_t* __restrict__ kk,
-                                                             int ksize, uint8_t* __restrict__ dst) {
-  const int wpr = (row_bytes + 3) >> 2;              // words per output row
-  const long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
-  const long long orow = idx / wpr;                  // b * OH + yy
-  if (orow >= n_rows) return;
-  const int o4 = (int)(idx - orow * wpr) * 4;
-  const long long b = orow / OH;
-  const int yy = (int)(orow - b * OH);
-  const int ymin = __ldg(bounds + 2 * yy), n = __ldg(bounds + 2 * yy + 1);
-  const int32_t* k = kk + (long long)yy * ksize;
-  const uint8_t* p = src + b * image_stride + (long long)ymin * pitch + o4;
-  uint8_t* out = dst + orow * (long long)row_bytes + o4;
-  const int n_out = min(4, row_bytes - o4);
+// One output word of the vertical pass: n_out (1..4) bytes at `out` from the n taps p, p + pitch, ... weighted by k.
+__device__ __forceinline__ void v_taps(const uint8_t* p, long long pitch, const int32_t* k, int n, int n_out, uint8_t* out) {
   int a0, a1, a2, a3;
   a0 = a1 = a2 = a3 = 1 << (kPrecisionBits - 1);
   const bool word_in = n_out == 4 && ((reinterpret_cast<uintptr_t>(p) | (uintptr_t)pitch) & 3u) == 0;
@@ -295,6 +279,27 @@ __global__ void __launch_bounds__(kThreads) resize_v_kernel(const uint8_t* __res
   } else {
     for (int t = 0; t < n_out; ++t) out[t] = (uint8_t)(packed >> (8 * t));
   }
+}
+
+// src: [B] images of H rows x row_bytes (pitch / image_stride in bytes); dst: [B, OH, row_bytes] contiguous.
+// One thread per 32-bit word of the output (flattened over rows, so narrow rows still fill the CTAs).
+__global__ void __launch_bounds__(kThreads) resize_v_kernel(const uint8_t* __restrict__ src, int row_bytes, long long pitch,
+                                                             long long image_stride, int OH, long long n_rows,
+                                                             const int32_t* __restrict__ bounds, const int32_t* __restrict__ kk,
+                                                             int ksize, uint8_t* __restrict__ dst) {
+  const int wpr = (row_bytes + 3) >> 2;              // words per output row
+  const long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
+  const long long orow = idx / wpr;                  // b * OH + yy
+  if (orow >= n_rows) return;
+  const int o4 = (int)(idx - orow * wpr) * 4;
+  const long long b = orow / OH;
+  const int yy = (int)(orow - b * OH);
+  const int ymin = __ldg(bounds + 2 * yy), n = __ldg(bounds + 2 * yy + 1);
+  const int32_t* k = kk + (long long)yy * ksize;
+  const uint8_t* p = src + b * image_stride + (long long)ymin * pitch + o4;
+  uint8_t* out = dst + orow * (long long)row_bytes + o4;
+  const int n_out = min(4, row_bytes - o4);
+  v_taps(p, pitch, k, n, n_out, out);
 }
 
 // Vertical pass, 16 output bytes per thread (rows and pitches that are multiples of 16 bytes: any OW % 16 == 0):
@@ -329,6 +334,148 @@ __global__ void __launch_bounds__(kThreads) resize_v16_kernel(const uint8_t* __r
   for (int j = 0; j < 4; ++j)
     o[j] = clip8(acc[4 * j]) | (clip8(acc[4 * j + 1]) << 8) | (clip8(acc[4 * j + 2]) << 16) | (clip8(acc[4 * j + 3]) << 24);
   *reinterpret_cast<uint4*>(dst + orow * (long long)row_bytes + o16) = make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// ---- ragged batches: every image has its own H x W, all go to OH x OW ---------------------------------------------
+// Three launches whatever the number of shapes: the coefficient tables of every image, the horizontal pass over the
+// rows of the images whose width changes, the vertical pass over all n * OH output rows.
+
+// Pillow's bicubic kernel (a = -0.5) in double precision, each operation rounded on its own as the host code's
+// (built with -ffp-contract=off): nvcc would otherwise fuse the multiply-adds and the tables would differ.
+__device__ __forceinline__ double bicubic_filter_dev(double x) {
+  if (x < 0.0) x = -x;
+  if (x < 1.0) return __dadd_rn(__dmul_rn(__dmul_rn(__dsub_rn(__dmul_rn(1.5, x), 2.5), x), x), 1.0);
+  if (x < 2.0) return __dmul_rn(__dsub_rn(__dmul_rn(__dadd_rn(__dmul_rn(__dsub_rn(x, 5.0), x), 8.0), x), 4.0), -0.5);
+  return 0.0;
+}
+
+// One thread per output position of either axis of every image (n x (OW + OH) threads): the bounds and kk rows of
+// gnc_resize_bicubic_coeffs, at the image's workspace offsets.  Axes that keep their size (ksize 0) have no table.
+__global__ void __launch_bounds__(kThreads) resize_ragged_tables_kernel(const gnc_resize_image_t* __restrict__ images,
+                                                                         long long n, int OH, int OW, int32_t* __restrict__ tables) {
+  const long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
+  const long long i = idx / (OW + OH);
+  if (i >= n) return;
+  int xx = (int)(idx - i * (OW + OH));
+  const gnc_resize_image_t* im = images + i;
+  int in_size, out_size, ksize;
+  long long tab;
+  if (xx < OW) {
+    in_size = im->width, out_size = OW, ksize = im->ksize_x, tab = im->tab_x;
+  } else {
+    xx -= OW;
+    in_size = im->height, out_size = OH, ksize = im->ksize_y, tab = im->tab_y;
+  }
+  if (ksize == 0) return;
+  const double scale = __ddiv_rn((double)in_size, (double)out_size);
+  const double filterscale = scale < 1.0 ? 1.0 : scale;
+  const double support = __dmul_rn(2.0, filterscale);
+  const double ss = __ddiv_rn(1.0, filterscale);
+  const double center = __dadd_rn(0.0, __dmul_rn(__dadd_rn((double)xx, 0.5), scale));
+  int xmin = (int)__dadd_rn(__dsub_rn(center, support), 0.5);
+  if (xmin < 0) xmin = 0;
+  int xmax = (int)__dadd_rn(__dadd_rn(center, support), 0.5);
+  if (xmax > in_size) xmax = in_size;
+  xmax -= xmin;
+  int32_t* bounds = tables + tab;
+  int32_t* k = bounds + 2 * out_size + (long long)xx * ksize;
+  double ww = 0.0;
+  for (int x = 0; x < xmax; ++x)
+    ww = __dadd_rn(ww, bicubic_filter_dev(__dmul_rn(__dadd_rn(__dsub_rn((double)(x + xmin), center), 0.5), ss)));
+  for (int x = 0; x < xmax; ++x) {
+    double v = bicubic_filter_dev(__dmul_rn(__dadd_rn(__dsub_rn((double)(x + xmin), center), 0.5), ss));
+    if (ww != 0.0) v = __ddiv_rn(v, ww);
+    v = __dmul_rn(v, (double)(1 << kPrecisionBits));
+    k[x] = v < 0 ? (int)__dadd_rn(-0.5, v) : (int)__dadd_rn(0.5, v);
+  }
+  for (int x = xmax; x < ksize; ++x) k[x] = 0;
+  bounds[2 * xx] = xmin;
+  bounds[2 * xx + 1] = xmax;
+}
+
+// Horizontal pass, one CTA per row of tmp [h_rows, OW, 3]: the rows of the images whose width changes, image after
+// image (tmp_row = running row count).  The row's image is the last one whose tmp_row is <= the row: images that
+// contribute no rows share their tmp_row with the next image, which the search then prefers.
+__global__ void __launch_bounds__(kThreads) resize_ragged_h_kernel(const gnc_resize_image_t* __restrict__ images, int n, int OW,
+                                                                    const int32_t* __restrict__ tables, uint8_t* __restrict__ tmp) {
+  extern __shared__ __align__(16) uint8_t s_row[];
+  __shared__ int s_image;
+  const long long row = blockIdx.x;
+  if (threadIdx.x == 0) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (images[mid].tmp_row <= row) lo = mid;
+      else hi = mid - 1;
+    }
+    s_image = lo;
+  }
+  __syncthreads();
+  const gnc_resize_image_t* im = images + s_image;
+  const uint8_t* g = im->src + (row - im->tmp_row) * im->pitch;
+  const int nbytes = 3 * im->width;
+  // the shared copy keeps the row's 16-byte phase, so that its aligned middle part moves as 128-bit words
+  const int phase = (int)(reinterpret_cast<uintptr_t>(g) & 15u);
+  uint8_t* s = s_row + phase;
+  const int head = min(nbytes, (16 - phase) & 15);
+  const int nvec = (nbytes - head) >> 4;
+  for (int i = threadIdx.x; i < head; i += kThreads) s[i] = g[i];
+  const uint4* gv = reinterpret_cast<const uint4*>(g + head);
+  uint4* sv = reinterpret_cast<uint4*>(s + head);
+  for (int i = threadIdx.x; i < nvec; i += kThreads) sv[i] = __ldg(gv + i);
+  for (int i = head + (nvec << 4) + threadIdx.x; i < nbytes; i += kThreads) s[i] = g[i];
+  __syncthreads();
+
+  const int ksize = im->ksize_x;
+  const int32_t* bounds = tables + im->tab_x;
+  const int32_t* kk = bounds + 2 * OW;
+  uint8_t* out = tmp + row * (3LL * OW);
+  for (int xx = threadIdx.x; xx < OW; xx += kThreads) {
+    const int xmin = __ldg(bounds + 2 * xx), nt = __ldg(bounds + 2 * xx + 1);
+    const int32_t* k = kk + (long long)xx * ksize;
+    const uint8_t* p = s + 3 * xmin;
+    int a0, a1, a2;
+    a0 = a1 = a2 = 1 << (kPrecisionBits - 1);
+    for (int x = 0; x < nt; ++x) {
+      const int c = __ldg(k + x);
+      a0 += (int)p[3 * x] * c;
+      a1 += (int)p[3 * x + 1] * c;
+      a2 += (int)p[3 * x + 2] * c;
+    }
+    out[3 * xx] = (uint8_t)clip8(a0);
+    out[3 * xx + 1] = (uint8_t)clip8(a1);
+    out[3 * xx + 2] = (uint8_t)clip8(a2);
+  }
+}
+
+// Vertical pass, one thread per 32-bit word of dst [n, OH, OW, 3].  An image reads its rows from tmp when its width
+// changed, else from its source; an image whose height is already OH copies row yy.
+__global__ void __launch_bounds__(kThreads) resize_ragged_v_kernel(const gnc_resize_image_t* __restrict__ images, long long n_rows,
+                                                                    int OH, int OW, const int32_t* __restrict__ tables,
+                                                                    const uint8_t* __restrict__ tmp, uint8_t* __restrict__ dst) {
+  const int row_bytes = 3 * OW;
+  const int wpr = (row_bytes + 3) >> 2;
+  const long long idx = (long long)blockIdx.x * kThreads + threadIdx.x;
+  const long long orow = idx / wpr;                  // i * OH + yy
+  if (orow >= n_rows) return;
+  const int o4 = (int)(idx - orow * wpr) * 4;
+  const long long i = orow / OH;
+  const int yy = (int)(orow - i * OH);
+  const gnc_resize_image_t* im = images + i;
+  const bool from_tmp = im->ksize_x != 0;
+  const uint8_t* src = from_tmp ? tmp + im->tmp_row * (long long)row_bytes : im->src;
+  const long long pitch = from_tmp ? (long long)row_bytes : im->pitch;
+  const int ksize = im->ksize_y;
+  uint8_t* out = dst + orow * (long long)row_bytes + o4;
+  const int n_out = min(4, row_bytes - o4);
+  if (ksize == 0) {
+    const uint8_t* p = src + (long long)yy * pitch + o4;
+    for (int t = 0; t < n_out; ++t) out[t] = p[t];
+    return;
+  }
+  const int32_t* bounds = tables + im->tab_y;
+  const int ymin = __ldg(bounds + 2 * yy), n = __ldg(bounds + 2 * yy + 1);
+  v_taps(src + (long long)ymin * pitch + o4, pitch, bounds + 2 * OH + (long long)yy * ksize, n, n_out, out);
 }
 
 // ---- coefficient tables (host; Pillow's precompute_coeffs + normalize_coeffs_8bpc, full box) --------------------
@@ -462,4 +609,32 @@ extern "C" int gnc_resize_bicubic_u8(const uint8_t* src, int64_t B, int H, int W
     if (rc != GNC_OK) return rc;
   }
   return GNC_OK;
+}
+
+extern "C" int gnc_resize_bicubic_ragged_u8(const gnc_resize_image_t* images, int64_t n, int OH, int OW, int64_t h_rows, int max_w,
+                                            int32_t* tables, uint8_t* tmp, uint8_t* dst, gnc_stream_t stream) {
+  GNC_REQUIRE(n >= 0 && OH > 0 && OW > 0 && h_rows >= 0 && max_w >= 0, "resize_bicubic_ragged: bad arguments");
+  if (n == 0) return GNC_OK;
+  GNC_REQUIRE(images && tables && dst, "resize_bicubic_ragged: images, tables and dst are required");
+  GNC_REQUIRE(h_rows == 0 || (tmp && max_w > 0), "resize_bicubic_ragged: tmp [h_rows, OW, 3] and max_w are required when a width changes");
+  GNC_REQUIRE(n < (1LL << 31) && h_rows < (1LL << 31), "resize_bicubic_ragged: too many images or rows for one launch");
+  const size_t smem = (size_t)3 * max_w + 32;
+  GNC_REQUIRE(smem <= 200 * 1024, "resize_bicubic_ragged: source rows wider than 68 000 pixels are not supported");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long tab_blocks = ceil_div(n * (long long)(OW + OH), (long long)rsz::kThreads);
+  const long long v_blocks = ceil_div(n * (long long)OH * ((3LL * OW + 3) >> 2), (long long)rsz::kThreads);
+  GNC_REQUIRE(tab_blocks < (1LL << 31) && v_blocks < (1LL << 31), "resize_bicubic_ragged: output too large for one launch");
+  rsz::resize_ragged_tables_kernel<<<(unsigned)tab_blocks, rsz::kThreads, 0, st>>>(images, n, OH, OW, tables);
+  int rc = check_launch("resize_ragged_tables_kernel");
+  if (rc != GNC_OK) return rc;
+  if (h_rows > 0) {
+    static SmemAttrOnce smem_attr;
+    if (smem > 48 * 1024)
+      if (int rc_attr = smem_attr.ensure(rsz::resize_ragged_h_kernel, 200 * 1024, "resize_bicubic_ragged")) return rc_attr;
+    rsz::resize_ragged_h_kernel<<<(unsigned)h_rows, rsz::kThreads, smem, st>>>(images, (int)n, OW, tables, tmp);
+    rc = check_launch("resize_ragged_h_kernel");
+    if (rc != GNC_OK) return rc;
+  }
+  rsz::resize_ragged_v_kernel<<<(unsigned)v_blocks, rsz::kThreads, 0, st>>>(images, n * (long long)OH, OH, OW, tables, tmp, dst);
+  return check_launch("resize_ragged_v_kernel");
 }

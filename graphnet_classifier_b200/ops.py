@@ -12,6 +12,7 @@ Operators (each with its backward wired through ``torch.autograd.Function``):
   gather_rows          x[row] / x[col]                                 PyG MetaLayer, models/GNN.py:146
   edge_geometry        [pos[col]-pos[row], L1]                         models/GNN.py:299-302
   resize_bicubic       PIL Image.resize((r, r)) on the device, bit-exact  utils/image_to_graph/image_to_graph_optimized.py:65-70
+  resize_bicubic_ragged  the same for a list of images of different sizes, in three launches
 """
 from __future__ import annotations
 
@@ -618,6 +619,70 @@ def resize_bicubic(images: Tensor, out_h: int, out_w: Optional[int] = None) -> T
     check(_call("resize_bicubic", 0.0, nbytes, _lib.load().gnc_resize_bicubic_u8, img.data_ptr(), B, H, W, pitch, istride,
                 out_h, out_w, _p(bx), _p(kx), ksx, _p(by), _p(ky), ksy, _p(tmp), dst.data_ptr(), _stream()), "resize_bicubic")
     return dst[0] if single else dst
+
+
+def _ragged_plan(heights, widths, out_h: int, out_w: int):
+    """Host half of ``resize_bicubic_ragged``, from the shapes alone: a ``gnc_resize_image`` record per image with its
+    taps per axis (0 where the size is already the target), its table offsets and its first row of the horizontal
+    pass's output.  Returns ``(records, table int32 elements, horizontal-pass rows, widest width changed)``; the
+    caller fills ``src`` and ``pitch``."""
+    import numpy as np
+    h = np.asarray(heights, np.int64)
+    w = np.asarray(widths, np.int64)
+
+    def taps(size, out):                    # gnc_resize_bicubic_ksize: ceil(2 max(in / out, 1)) * 2 + 1
+        return np.where(size != out, np.ceil(2.0 * np.maximum(size / out, 1.0)).astype(np.int64) * 2 + 1, 0)
+
+    kx, ky = taps(w, out_w), taps(h, out_h)
+    x_len = np.where(kx > 0, out_w * (2 + kx), 0)
+    y_len = np.where(ky > 0, out_h * (2 + ky), 0)
+    tab_x = np.cumsum(x_len + y_len) - (x_len + y_len)
+    h_rows = np.where(kx > 0, h, 0)
+    rec = np.zeros(len(h), np.dtype(_lib.GncResizeImage))
+    rec["height"], rec["width"], rec["ksize_x"], rec["ksize_y"] = h, w, kx, ky
+    rec["tab_x"], rec["tab_y"] = tab_x, tab_x + x_len
+    rec["tmp_row"] = np.cumsum(h_rows) - h_rows
+    max_w = int(w[kx > 0].max()) if (kx > 0).any() else 0
+    return rec, int((x_len + y_len).sum()), int(h_rows.sum()), max_w
+
+
+def resize_bicubic_ragged(images: Sequence[Tensor], out_h: int, out_w: Optional[int] = None) -> Tensor:
+    """``PIL.Image.resize((out_w, out_h))`` of every image of a list of CUDA ``uint8 [H_i, W_i, 3]`` tensors of any
+    sizes (strided views too) -> ``uint8 [n, out_h, out_w, 3]``, bit-identical to ``resize_bicubic`` of each image.
+    Three launches whatever the number of shapes: the coefficient tables are computed on the device, and the image
+    records reach it in one copy from pinned memory.  ``resize_bicubic`` stays the form for batches of one shape."""
+    import numpy as np
+    out_w = out_h if out_w is None else out_w
+    if out_h <= 0 or out_w <= 0:
+        raise ValueError(f"resize_bicubic_ragged: bad output size {out_h} x {out_w}")
+    n = len(images)
+    if n == 0:
+        dev = torch.device("cuda", torch.cuda.current_device())
+        return torch.empty(0, out_h, out_w, 3, dtype=torch.uint8, device=dev)
+    _require_cuda(*images)
+    dev = images[0].device
+    srcs = []
+    for t in images:
+        if t.dtype != torch.uint8 or t.dim() != 3 or t.shape[2] != 3 or t.shape[0] == 0 or t.shape[1] == 0:
+            raise ValueError(f"resize_bicubic_ragged expects uint8 [H, W, 3] images, got {t.dtype} {tuple(t.shape)}")
+        if t.device != dev:
+            raise ValueError(f"resize_bicubic_ragged: images on {t.device} and {dev}")
+        if t.stride(2) != 1 or (t.shape[1] > 1 and t.stride(1) != 3):
+            t = t.contiguous()
+        srcs.append(t)
+    rec, n_tables, h_rows, max_w = _ragged_plan([t.shape[0] for t in srcs], [t.shape[1] for t in srcs], out_h, out_w)
+    rec["src"] = [t.data_ptr() for t in srcs]
+    rec["pitch"] = [t.stride(0) if t.shape[0] > 1 else 3 * t.shape[1] for t in srcs]
+    host = torch.empty(rec.nbytes, dtype=torch.uint8, pin_memory=True)
+    host.numpy()[:] = rec.view(np.uint8)
+    records = host.to(dev, non_blocking=True)       # the host allocator keeps `host` until this copy has run
+    tables = torch.empty(max(n_tables, 1), dtype=torch.int32, device=dev)
+    tmp = torch.empty(h_rows * 3 * out_w, dtype=torch.uint8, device=dev) if h_rows else None
+    dst = torch.empty(n, out_h, out_w, 3, dtype=torch.uint8, device=dev)
+    nbytes = 3.0 * (sum(t.shape[0] * t.shape[1] for t in srcs) + n * out_h * out_w)
+    check(_call("resize_bicubic_ragged", 0.0, nbytes, _lib.load().gnc_resize_bicubic_ragged_u8, records.data_ptr(), n, out_h,
+                out_w, h_rows, max_w, tables.data_ptr(), _p(tmp), dst.data_ptr(), _stream()), "resize_bicubic_ragged")
+    return dst
 
 
 class _ScatterSumFn(torch.autograd.Function):

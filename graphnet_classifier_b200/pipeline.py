@@ -67,11 +67,16 @@ class GraphClassifierPipeline:
     def _to_device(self, images) -> Tensor:
         """``uint8 [B, r, r, 3]`` on the device.  Images of another size (one ``[B, H, W, 3]`` array, or a
         list of differently sized ``[H, W, 3]`` arrays, e.g. decoded files) are resized on the device exactly
-        as the reference's ``image.resize((r, r))`` does (``ops.resize_bicubic``)."""
+        as the reference's ``image.resize((r, r))`` does (``ops.resize_bicubic``; a list in one
+        ``ops.resize_bicubic_ragged`` call)."""
         r = self.resize_value
         if isinstance(images, (list, tuple)):
-            parts = [self._to_device(im) for im in images]
-            return parts[0] if len(parts) == 1 else torch.cat(parts, 0)
+            parts = []
+            for im in images:
+                t = im if isinstance(im, Tensor) else torch.as_tensor(im)
+                t = t if t.is_cuda else t.to(self.device, non_blocking=True)
+                parts.extend([t] if t.dim() == 3 else t.unbind(0))
+            return ops.resize_bicubic_ragged(parts, r, r)
         t = images if isinstance(images, Tensor) else torch.as_tensor(images)
         if t.dim() == 3:
             t = t.unsqueeze(0)

@@ -13,8 +13,9 @@ utils/image_to_graph/image_to_graph_optimized.py:65-70, utils/inference.py:47). 
   process) are decoded on a thread pool instead;
 * images of one shape travel as ONE host->device copy on a copy stream; two staging buffers alternate, so the pool
   decodes chunk ``i + 1`` while chunk ``i`` is copied and consumed;
-* the resize is the Pillow-exact device kernel (``ops.resize_bicubic``), so the pixels that reach the graph builder are
-  bit for bit the reference's.
+* the resize is the Pillow-exact device kernel, so the pixels that reach the graph builder are bit for bit the
+  reference's: ``ops.resize_bicubic`` when a chunk holds one shape, else one ``ops.resize_bicubic_ragged`` call over
+  all its images, whatever the number of shapes.
 
 """
 from __future__ import annotations
@@ -188,23 +189,12 @@ class DecodePool:
         self.stats["host_decoded"] += len(host)
         for i, a in host.items():
             imgs[i] = torch.from_numpy(np.array(a, dtype=np.uint8)).to(self.device)
-        groups = {}
-        for i, t in enumerate(imgs):
-            groups.setdefault(tuple(t.shape), []).append(i)
-        n = len(imgs)
-        out = None
-        for shape, idxs in groups.items():
-            if len(idxs) == n and all(imgs[i].data_ptr() + imgs[i].numel() == imgs[i + 1].data_ptr() for i in range(n - 1)):
-                batch = torch.as_strided(imgs[0], (n, *shape), (imgs[0].numel(), shape[1] * 3, 3, 1))     # already packed
-            else:
-                batch = torch.stack([imgs[i] for i in idxs])
-            px = batch if (shape[0] == r and shape[1] == r) else ops.resize_bicubic(batch, r, r)
-            if len(groups) == 1:
-                return px
-            if out is None:
-                out = torch.empty(n, r, r, 3, dtype=torch.uint8, device=self.device)
-            out[torch.as_tensor(idxs, device=self.device)] = px
-        return out
+        n, shape = len(imgs), imgs[0].shape
+        if all(t.shape == shape for t in imgs) and all(
+                imgs[i].data_ptr() + imgs[i].numel() == imgs[i + 1].data_ptr() for i in range(n - 1)):
+            batch = torch.as_strided(imgs[0], (n, *shape), (imgs[0].numel(), shape[1] * 3, 3, 1))     # already packed
+            return batch if (shape[0] == r and shape[1] == r) else ops.resize_bicubic(batch, r, r)
+        return ops.resize_bicubic_ragged(imgs, r, r)
 
     def _decode_chunk(self, items: Sequence, slot: int):
         """Decodes ``items`` on the pool; returns ``[(shape, indices, pinned view [k, H, W, 3])]`` grouped by shape."""
@@ -257,14 +247,16 @@ class DecodePool:
             ev.record(self.copy_stream)
         self._events[slot] = ev
         cur.wait_event(ev)
-        out = torch.empty(n, r, r, 3, dtype=torch.uint8, device=self.device)
-        for idxs, dev_imgs in parts:
+        for _, dev_imgs in parts:
             dev_imgs.record_stream(cur)
-            px = dev_imgs if (dev_imgs.shape[1] == r and dev_imgs.shape[2] == r) else ops.resize_bicubic(dev_imgs, r, r)
-            if len(parts) == 1:
-                return px
-            out[torch.as_tensor(idxs, device=self.device)] = px
-        return out
+        if len(parts) == 1:
+            dev_imgs = parts[0][1]
+            return dev_imgs if (dev_imgs.shape[1] == r and dev_imgs.shape[2] == r) else ops.resize_bicubic(dev_imgs, r, r)
+        imgs = [None] * n
+        for idxs, dev_imgs in parts:
+            for i, im in zip(idxs, dev_imgs):
+                imgs[i] = im
+        return ops.resize_bicubic_ragged(imgs, r, r)
 
     # -- public ------------------------------------------------------------------------
     def stage(self, items: Sequence, resize_value: int) -> Tensor:

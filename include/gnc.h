@@ -263,6 +263,27 @@ int gnc_resize_bicubic_u8(const uint8_t* src, int64_t B, int H, int W, int64_t s
                           int OH, int OW, const int32_t* bounds_x, const int32_t* kk_x, int ksize_x,
                           const int32_t* bounds_y, const int32_t* kk_y, int ksize_y, uint8_t* tmp, uint8_t* dst,
                           gnc_stream_t stream);
+/* Ragged batches: n images, each of its own H x W, -> dst uint8 [n, OH, OW, 3] contiguous, in three launches whatever
+ * the number of shapes; bit-identical to resizing each image on its own.
+ *   images   DEVICE array of n descriptors.  The caller fills, from the shapes alone:
+ *              ksize_x / ksize_y  gnc_resize_bicubic_ksize of the axis, 0 when its size already is OW / OH;
+ *              tab_x / tab_y      int32 offsets into `tables` of the axis's bounds [out, 2] followed by its kk
+ *                                 [out, ksize]; non-overlapping (out * (2 + ksize) int32 each, none for ksize 0);
+ *              tmp_row            rows of tmp [h_rows, OW, 3] before this image: the running sum of height over the
+ *                                 images before it whose width changes.
+ *   h_rows   rows of tmp = the sum of height over the images whose width changes; max_w = their largest width.
+ *   tables   int32 workspace, written here (gnc_resize_bicubic_coeffs's tables, computed on the device).
+ * Sources may have any alignment and row pitch (pixels 3 bytes apart). */
+typedef struct gnc_resize_image {
+  const uint8_t* src;     /* [height, width, 3], rows `pitch` bytes apart */
+  int64_t pitch;
+  int64_t tmp_row;
+  int64_t tab_x, tab_y;
+  int32_t height, width;
+  int32_t ksize_x, ksize_y;
+} gnc_resize_image_t;
+int gnc_resize_bicubic_ragged_u8(const gnc_resize_image_t* images, int64_t n, int OH, int OW, int64_t h_rows, int max_w,
+                                 int32_t* tables, uint8_t* tmp, uint8_t* dst, gnc_stream_t stream);
 
 /* Stable CSR of edge ids grouped by key (= edge_index row 0 or row 1): the order
  * index_add_ visits edges in (models/GNN.py:20).  key is read with an element
