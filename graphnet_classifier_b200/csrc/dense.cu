@@ -628,7 +628,6 @@ __global__ void __launch_bounds__(256) layernorm_fwd_vec_kernel(const float* __r
   const int D4 = D >> 2;
   const long long warp_global = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long warps_total = ((long long)gridDim.x * blockDim.x) >> 5;
-  const float invD = 1.0f / (float)D;
   float4 g[VPL], bt[VPL];
 #pragma unroll
   for (int q = 0; q < VPL; ++q) {
@@ -658,7 +657,7 @@ __global__ void __launch_bounds__(256) layernorm_fwd_vec_kernel(const float* __r
       for (int q = 0; q < VPL; ++q) s += (v[t][q].x + v[t][q].y) + (v[t][q].z + v[t][q].w);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-      const float mu = s * invD;
+      const float mu = s / (float)D;      // (a division: exact for a constant row whatever D)
       float ss = 0.f;
 #pragma unroll
       for (int q = 0; q < VPL; ++q) {
@@ -670,7 +669,7 @@ __global__ void __launch_bounds__(256) layernorm_fwd_vec_kernel(const float* __r
       }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-      const float rs = 1.0f / sqrtf(ss * invD + eps);
+      const float rs = 1.0f / sqrtf(ss / (float)D + eps);
       if (lane == 0) {
         if (mean) mean[r] = mu;
         if (rstd) rstd[r] = rs;
@@ -701,19 +700,25 @@ __global__ void __launch_bounds__(256) layernorm_fwd_scalar_kernel(const float* 
   const int lane = threadIdx.x & 31;
   const long long warp_global = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long warps_total = ((long long)gridDim.x * blockDim.x) >> 5;
-  const float invD = 1.0f / (float)D;
   for (long long r = warp_global; r < M; r += warps_total) {
     const float* zr = z + r * ldz;
     float s = 0.f;
     for (int c = lane; c < D; c += 32) s += zr[c];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    const float mu = s * invD;
-    float ss = 0.f;
-    for (int c = lane; c < D; c += 32) { const float a = zr[c] - mu; ss += a * a; }
+    float mu = s / (float)D;
+    // corrected two-pass: the deviations from the first mean also sum to D times its rounding error, which matters when
+    // the row's centre is far from zero against its spread
+    float sd = 0.f, ss = 0.f;
+    for (int c = lane; c < D; c += 32) { const float a = zr[c] - mu; sd += a; ss += a * a; }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    const float rs = 1.0f / sqrtf(ss * invD + eps);
+    for (int o = 16; o > 0; o >>= 1) {
+      sd += __shfl_xor_sync(0xffffffffu, sd, o);
+      ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    }
+    const float dm = sd / (float)D;
+    mu += dm;
+    const float rs = 1.0f / sqrtf(fmaxf(ss / (float)D - dm * dm, 0.f) + eps);
     if (lane == 0) {
       if (mean) mean[r] = mu;
       if (rstd) rstd[r] = rs;

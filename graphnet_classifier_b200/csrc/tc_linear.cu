@@ -491,9 +491,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_linear_kernel(const Params p) 
         const long long g = wrow0 + lane;
         if (g < p.M) Ysel[g * p.ldy] = acc + (p.dot_b ? __ldg(p.dot_b) : 0.f);
       } else {
-        // LayerNorm.  Pass 1 over the accumulator: shifted one-pass statistics (shift = first
-        // element of the row, so the cancellation in E[d^2] - E[d]^2 is of order std^2);
-        // pass 2 re-reads TMEM, normalises and stores.  No 128-register row buffer.
+        // LayerNorm.  Pass 1 over the accumulator: each 32-column chunk's mean and sum of squared
+        // deviations from it (two sweeps over the chunk's registers), merged into the row's running
+        // mean / M2 with Chan's pairwise update.  Every term is a deviation from a mean, so the
+        // statistics are exact to fp32 rounding whatever the row's centre (a one-pass
+        // E[z^2] - E[z]^2, even shifted by the first element, loses ~7 bits when that element
+        // is an outlier of the row).  Pass 2 re-reads TMEM, normalises and stores.  No 128-register
+        // row buffer.
         float4 res[8];
         long long rrow[8];                              // residual rows: identity, or a table lookup
 #pragma unroll
@@ -505,23 +509,33 @@ __global__ void __launch_bounds__(kThreads, 1) tc_linear_kernel(const Params p) 
         }
         mbar_wait(d_full(eg), dph);
         tc_fence_after();
-        float shift = 0.f, s1 = 0.f, s2 = 0.f;
+        float mu = 0.f, m2 = 0.f;
 #pragma unroll 1
         for (int ch = 0; ch < 4; ++ch) {
           float r[32];
           tmem_ld32(taddr + ch * 32, r);
           tmem_ld_wait();
-          if (ch == 0) shift = r[0] + s_bias[0];
+          float s = 0.f;
 #pragma unroll
           for (int cidx = 0; cidx < 32; ++cidx) {
-            const float dlt = (r[cidx] + s_bias[ch * 32 + cidx]) - shift;
-            s1 += dlt;
-            s2 = fmaf(dlt, dlt, s2);
+            r[cidx] += s_bias[ch * 32 + cidx];
+            s += r[cidx];
           }
+          const float mc = s * (1.0f / 32);
+          float q = 0.f;
+#pragma unroll
+          for (int cidx = 0; cidx < 32; ++cidx) {
+            const float dlt = r[cidx] - mc;
+            q = fmaf(dlt, dlt, q);
+          }
+          // merge (32 ch columns, mean mu, M2 m2) with (32 columns, mean mc, M2 q)
+          const float delta = mc - mu;
+          const float inv_n = ch == 0 ? 1.0f : ch == 1 ? 0.5f : ch == 2 ? 1.0f / 3 : 0.25f;     // 1 / (ch + 1)
+          const float w = ch == 0 ? 0.0f : ch == 1 ? 16.0f : ch == 2 ? 64.0f / 3 : 24.0f;    // 32 ch / (ch + 1)
+          mu = fmaf(delta, inv_n, mu);
+          m2 += fmaf(delta * delta, w, q);
         }
-        const float m1 = s1 * (1.0f / kD);
-        const float mu = shift + m1;
-        const float var = fmaxf(s2 * (1.0f / kD) - m1 * m1, 0.f);
+        const float var = m2 * (1.0f / kD);
         const float rs = 1.0f / sqrtf(var + p.eps);
         if (p.ln_mean && wrow0 + lane < p.M) {          // thread = row: the statistics the backward reuses
           p.ln_mean[wrow0 + lane] = mu;

@@ -42,12 +42,21 @@ __global__ void __launch_bounds__(256) cross_entropy_kernel(const float* __restr
   }
 }
 
-// torch.optim.Adam's update (amsgrad off, weight decay off), one element per thread, 128-bit accesses:
-//   m = m + (g - m) (1 - b1);  v = v b2 + (1 - b2) g g;  p -= (lr / bc1) m / (sqrt(v) / sqrt(bc2) + eps)
+// torch.optim.Adam's update (amsgrad off, weight decay off), one element per thread, 128-bit accesses, with the
+// roundings of its default (foreach) CUDA path, so that the parameters come out bit for bit as torch's:
+//   m = fma(1 - b1, g - m, m);  v = fma(1 - b2, g g, round(v b2));  p = fma(-lr / bc1, m / (sqrt(v) / sqrt(bc2) + eps), p)
+// (every other step is rounded on its own: torch runs them as separate foreach kernels)
+__device__ __forceinline__ void adam_elem(float& p, float& m, float& v, float g, float one_minus_b1, float b2, float one_minus_b2,
+                                          float neg_step_size, float bc2_sqrt, float eps) {
+  m = __fmaf_rn(one_minus_b1, __fsub_rn(g, m), m);
+  v = __fmaf_rn(one_minus_b2, __fmul_rn(g, g), __fmul_rn(v, b2));
+  p = __fmaf_rn(neg_step_size, __fdiv_rn(m, __fadd_rn(__fdiv_rn(__fsqrt_rn(v), bc2_sqrt), eps)), p);
+}
+
 __global__ void __launch_bounds__(256) adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                         float* __restrict__ v, long long n4, long long n, float grad_scale,
-                                                        float one_minus_b1, float b2, float one_minus_b2, float step_size,
-                                                        float inv_bc2_sqrt, float eps) {
+                                                        float one_minus_b1, float b2, float one_minus_b2, float neg_step_size,
+                                                        float bc2_sqrt, float eps) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n4) {
     float4 pv = reinterpret_cast<float4*>(p)[i], mv = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
@@ -56,18 +65,13 @@ __global__ void __launch_bounds__(256) adam_step_kernel(float* __restrict__ p, c
     float* pp = &pv.x; float* mp = &mv.x; float* vp = &vv.x;
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
-      mp[c] = mp[c] + (gs[c] - mp[c]) * one_minus_b1;
-      vp[c] = vp[c] * b2 + one_minus_b2 * gs[c] * gs[c];
-      pp[c] = pp[c] - step_size * (mp[c] / (sqrtf(vp[c]) * inv_bc2_sqrt + eps));
+      adam_elem(pp[c], mp[c], vp[c], gs[c], one_minus_b1, b2, one_minus_b2, neg_step_size, bc2_sqrt, eps);
     }
     reinterpret_cast<float4*>(p)[i] = pv; reinterpret_cast<float4*>(m)[i] = mv; reinterpret_cast<float4*>(v)[i] = vv;
   }
   if (i == 0) {                                                // the n % 4 tail
     for (long long j = n4 * 4; j < n; ++j) {
-      const float gj = g[j] * grad_scale;
-      m[j] = m[j] + (gj - m[j]) * one_minus_b1;
-      v[j] = v[j] * b2 + one_minus_b2 * gj * gj;
-      p[j] = p[j] - step_size * (m[j] / (sqrtf(v[j]) * inv_bc2_sqrt + eps));
+      adam_elem(p[j], m[j], v[j], g[j] * grad_scale, one_minus_b1, b2, one_minus_b2, neg_step_size, bc2_sqrt, eps);
     }
   }
 }
@@ -95,13 +99,13 @@ int gnc_adam_step_f32(float* param, const float* grad, float* exp_avg, float* ex
   // (hyper-parameters arrive as doubles: torch forms 1 - beta in double before rounding to float, and
   // 1 - float(0.999) differs from float(1 - 0.999) by 1.3e-5 relative)
   const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
-  const float step_size = (float)(lr / bc1);
-  const float inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
+  const float neg_step_size = (float)(-(lr / bc1));
+  const float bc2_sqrt = (float)pow(bc2, 0.5);
   const long long n4 = n / 4;
   long long blocks = ceil_div<long long>(n4 > 0 ? n4 : 1, 256);
   adam_step_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, n4, n, grad_scale,
-                                                                       (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), step_size,
-                                                                       inv_bc2_sqrt, (float)eps);
+                                                                       (float)(1.0 - beta1), (float)beta2, (float)(1.0 - beta2), neg_step_size,
+                                                                       bc2_sqrt, (float)eps);
   return check_launch("adam_step_kernel");
 }
 

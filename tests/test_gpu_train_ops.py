@@ -43,6 +43,7 @@ def test_adam_step_matches_torch_adam():
         opt.step()
         ops.adam_step(p, grad * 4.0, m, v, step, lr=1e-3, grad_scale=0.25)
         assert float((p - ref.detach()).abs().max()) < 1e-6, step          # 1-2 ulp of weights of magnitude ~3
+        assert torch.equal(p, ref.detach()), step                           # torch's roundings, bit for bit
     st = opt.state[ref]
     rel = lambda a, b: float((a.double() - b.double()).norm() / b.double().norm())
     assert rel(m, st["exp_avg"]) < 1e-6 and rel(v, st["exp_avg_sq"]) < 1e-6
