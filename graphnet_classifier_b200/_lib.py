@@ -87,6 +87,17 @@ class GncJpegChain(Structure):
 
 GNC_JPEG_MAX_SCANS, GNC_JPEG_MAX_TABLES = 64, 32
 
+GNC_UNSUPPORTED = GNC_JPEG_UNSUPPORTED
+GNC_PNG_MAX_RAW_BYTES = 2 << 20
+
+
+class GncPngImage(Structure):
+    """struct gnc_png_image (include/gnc.h)."""
+    _fields_ = [("width", c_int32), ("height", c_int32), ("color_type", c_int32), ("bit_depth", c_int32),
+                ("row_bytes", c_int32), ("bpp", c_int32), ("window", c_int32), ("_pad", c_int32),
+                ("stream_offset", c_int64), ("stream_bytes", c_int64), ("raw_offset", c_int64), ("raw_bytes", c_int64),
+                ("pixel_offset", c_int64), ("palette", (c_uint8 * 3) * 256)]
+
 
 class GncResizeImage(Structure):
     """struct gnc_resize_image (include/gnc.h)."""
@@ -188,6 +199,8 @@ SIGNATURES = {
                                           _P]),
     "gnc_jpeg_decode_progressive_rgb_u8": (c_int, [_P, _P, c_int, _P, _P, c_int, _P, c_int64, c_int64, _P, _P, _P, _P]),
     "gnc_debug_jpeg_chains_per_warp": (c_int, [c_int]),
+    "gnc_png_pack": (c_int, [_P, _P, c_int, c_int, _P, c_int64, _P, _P, _P]),
+    "gnc_png_decode_rgb_u8": (c_int, [_P, _P, c_int, _P, _P, _P, _P]),
     "gnc_tc_bwd_layer_parts": (c_int32, [c_int64]),
     "gnc_tc_bwd_reduce_batch_f32": (c_int, [POINTER(GncBwdReduceItem), c_int32, _P]),
 }

@@ -15,7 +15,7 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libgnc.so")
-SOURCES = ["graph_build.cu", "aggregate.cu", "dense.cu", "tc_linear.cu", "tc_chain.cu", "tc_wgrad.cu", "tc_bwd.cu", "train_ops.cu", "narrow.cu", "slic.cu", "slic_connect.cu", "resize.cu", "jpeg.cu"]
+SOURCES = ["graph_build.cu", "aggregate.cu", "dense.cu", "tc_linear.cu", "tc_chain.cu", "tc_wgrad.cu", "tc_bwd.cu", "train_ops.cu", "narrow.cu", "slic.cu", "slic_connect.cu", "resize.cu", "jpeg.cu", "png.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17",
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -37,5 +37,10 @@ def decode_into(args):
     return h, w, None
 
 
+def decode(path):
+    """``Image.open(path).convert('RGB')`` as an array, returned through the pipe."""
+    return np.asarray(Image.open(path).convert("RGB"), dtype=np.uint8)
+
+
 def warm(_):
     return True

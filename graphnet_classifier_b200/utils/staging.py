@@ -5,7 +5,9 @@ utils/image_to_graph/image_to_graph_optimized.py:65-70, utils/inference.py:47). 
 * baseline JPEG files are decoded ON THE DEVICE (``utils/jpeg.py``, csrc/jpeg.cu: libjpeg's integer algorithm restated,
   bit for bit Pillow's pixels): the pool's threads only read the files and parse their markers, and only the compressed
   bytes cross PCIe; with ``device_jpeg="progressive"`` progressive JPEG files are decoded on the device too;
-* everything else (PNG, progressive / CMYK JPEG, ...; or all files with ``device_jpeg=False``): the decode
+* with ``device_png=True`` PNG files are decoded on the device as well (``utils/png.py``, csrc/png.cu: bit for bit
+  Pillow's pixels), whatever ``device_jpeg`` says about JPEG files;
+* everything else (PNG unless asked for, progressive / CMYK JPEG, ...; or all files with ``device_jpeg=False``): the decode
   (``Image.open`` + ``convert('RGB')``: libjpeg inside Pillow) runs on a pool of host PROCESSES (Pillow's
   Python-level file handling holds the GIL for about half of a small file's decode time: 8 threads give 2 x one
   thread, processes scale with the cores), each image decoded straight into its slot of a shared-memory staging
@@ -30,6 +32,9 @@ from PIL import Image
 from torch import Tensor
 
 from .. import ops
+
+
+_JPEG_MAGIC, _PNG_MAGIC = b"\xff\xd8", b"\x89PNG\r\n\x1a\n"
 
 
 def _decode(path_or_image) -> np.ndarray:
@@ -68,7 +73,7 @@ class DecodePool:
     ``processes=False`` use the thread pool."""
 
     def __init__(self, workers: Optional[int] = None, device=None, processes: bool = True, slot_bytes: int = 1 << 20,
-                 device_jpeg="auto"):
+                 device_jpeg="auto", device_png: bool = False):
         self.workers = int(workers) if workers else max(1, (os.cpu_count() or 2) - 1)
         self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         if self.device.type != "cuda":
@@ -90,6 +95,12 @@ class DecodePool:
         self.device_jpeg = bool(device_jpeg)
         self._jpeg_staging = [{}, {}]
         self.stats = {"device_jpeg": 0, "host_decoded": 0}
+        # PNG files: inflate, unfilter and conversion on the GPU, opt-in; files the device leaves out or finds damaged
+        # take the host path, which gives Pillow's pixels or Pillow's exception
+        self.device_png = bool(device_png)
+        self._png_staging = [{}, {}]
+        if self.device_png:
+            self.stats["device_png"] = 0
 
     def _process_pool(self):
         if self._procs is None:
@@ -157,10 +168,19 @@ class DecodePool:
             groups[(h, w, 3)][1].append(view)
         return [(shape, idxs, views) for shape, (idxs, views) in groups.items()]
 
+    def _host_decode(self, paths: Sequence) -> list:
+        """Pillow on the host for the files of a device-decode chunk the device does not take: on the worker processes
+        when the pool decodes JPEGs on the host (``device_jpeg=False`` with ``device_png=True``: those JPEGs stay on the
+        processes they would take without ``device_png``), else on the thread pool."""
+        if self.processes and not self.device_jpeg:
+            from . import _decode_worker
+            return list(self._process_pool().map(_decode_worker.decode, [str(p) for p in paths],
+                                                 chunksize=max(1, len(paths) // (4 * self.workers))))
+        return list(self.pool.map(_decode, paths))
+
     def _read_chunk_jpeg(self, paths: Sequence, slot: int):
-        """Device-JPEG form of a chunk: the pool's threads read the files and parse their markers (the C parser
-        releases the GIL); files the device decoder does not cover are decoded by Pillow here, on the host."""
-        from . import jpeg as gjpeg
+        """Device-decode form of a chunk (device JPEG and / or PNG): the pool's threads read the files (the C packers
+        release the GIL); files of no format the device decodes are decoded by Pillow here, on the host."""
 
         def read(path):
             with open(path, "rb") as f:
@@ -169,8 +189,9 @@ class DecodePool:
         datas = list(self.pool.map(read, paths))
         # which files the device decoder covers is known only after the pack step (on upload); files it rejects are
         # decoded here by Pillow when their magic is not JPEG's, and after the device call otherwise
-        rest = [i for i, d in enumerate(datas) if d[:2] != b"\xff\xd8"]
-        host = dict(zip(rest, self.pool.map(_decode, [paths[i] for i in rest]))) if rest else {}
+        rest = [i for i, d in enumerate(datas) if not ((self.device_jpeg and d[:2] == _JPEG_MAGIC) or
+                                                        (self.device_png and d[:8] == _PNG_MAGIC))]
+        host = dict(zip(rest, self._host_decode([paths[i] for i in rest]))) if rest else {}
         pairs = [(d, None) for d in datas]
         return {"jpeg": pairs, "host": host, "slot": slot, "paths": list(paths)}
 
@@ -179,13 +200,27 @@ class DecodePool:
         r = int(resize_value)
         pairs, host = chunk["jpeg"], chunk["host"]
         datas = [d if i not in host else b"" for i, (d, _) in enumerate(pairs)]
-        imgs = gjpeg.decode_batch(datas, self.device, staging=self._jpeg_staging[chunk["slot"]],
-                                  progressive=self.progressive_jpeg)
-        late = [i for i, t in enumerate(imgs) if t is None and i not in host]     # JPEGs outside the device decoder's scope
+        png = [i for i, d in enumerate(datas) if self.device_png and d[:8] == _PNG_MAGIC]
+        if self.device_jpeg:
+            jpeg_datas = [b"" if d[:8] == _PNG_MAGIC else d for d in datas] if png else datas
+            imgs = gjpeg.decode_batch(jpeg_datas, self.device, staging=self._jpeg_staging[chunk["slot"]],
+                                      progressive=self.progressive_jpeg)
+        else:
+            imgs = [None] * len(datas)
+        n_png = 0
+        if png:
+            from . import png as gpng
+            for i, t in zip(png, gpng.decode_batch([datas[i] for i in png], self.device,
+                                                   staging=self._png_staging[chunk["slot"]])):
+                imgs[i] = t
+                n_png += t is not None
+        late = [i for i, t in enumerate(imgs) if t is None and i not in host]     # files outside the device decoders' scope
         if late:
             host = dict(host)
-            host.update(zip(late, self.pool.map(_decode, [chunk["paths"][i] for i in late])))
-        self.stats["device_jpeg"] += len(imgs) - len(host)
+            host.update(zip(late, self._host_decode([chunk["paths"][i] for i in late])))
+        self.stats["device_jpeg"] += len(imgs) - len(host) - n_png
+        if self.device_png:
+            self.stats["device_png"] += n_png
         self.stats["host_decoded"] += len(host)
         for i, a in host.items():
             imgs[i] = torch.from_numpy(np.array(a, dtype=np.uint8)).to(self.device)
@@ -198,7 +233,7 @@ class DecodePool:
 
     def _decode_chunk(self, items: Sequence, slot: int):
         """Decodes ``items`` on the pool; returns ``[(shape, indices, pinned view [k, H, W, 3])]`` grouped by shape."""
-        if self.device_jpeg and items and all(isinstance(it, (str, os.PathLike)) for it in items):
+        if (self.device_jpeg or self.device_png) and items and all(isinstance(it, (str, os.PathLike)) for it in items):
             return self._read_chunk_jpeg(items, slot)
         if self._events[slot] is not None:
             self._events[slot].synchronize()            # the previous copy out of this buffer is done

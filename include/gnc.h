@@ -244,6 +244,44 @@ int gnc_jpeg_decode_progressive_rgb_u8(const uint8_t* stream, const gnc_jpeg_ima
 /* Debug aid: chains per warp of the progressive entropy kernel (1..32; anything else = the default, 1).  Same result. */
 int gnc_debug_jpeg_chains_per_warp(int n);
 
+/* PNG files, bit for bit  np.asarray(Image.open(f).convert('RGB'))  with Pillow 12 (csrc/png.cu, csrc/inflate.h):
+ * non-interlaced grey 1 / 2 / 4 / 8 / 16, RGB 8 / 16, palette 1 / 2 / 4 / 8, grey + alpha 8 / 16 and RGBA 8 / 16 bit;
+ * alpha is dropped, 16-bit samples give their high byte except 16-bit grey (I;16), which saturates at 255, 1 / 2 / 4-bit
+ * grey is scaled by 255 / 85 / 17, palette indices past the PLTE (or without one) give black.
+ * gnc_png_pack (HOST): parses a batch on `threads` host threads.  Per file that is in: images_out[j] with geometry,
+ *   palette, window, stream_offset (the file's IDAT payloads, back to back in stream_out: pinned memory, capacity >= sum
+ *   of sizes), raw_offset / raw_bytes (its filtered rows, height * (1 + row_bytes)) and pixel_offset (running sum of
+ *   width * height); index_out[j] = index of that file in `datas`.  Files are ordered longest stream first.
+ *   Left out: Adam7 interlacing, APNG, unknown critical chunks, a CRC mismatch on any chunk but IDAT, non-consecutive
+ *   IDATs, iCCP / zTXt / iTXt chunks, ancillary chunks too short for Pillow's reader (tRNS, gAMA, sRGB, pHYs, a cHRM
+ *   that is not whole 4-byte values), a zlib header other than method 8 / CINFO <= 7 / no preset dictionary, raw data
+ *   above GNC_PNG_MAX_RAW_BYTES, and anything that does not parse as whole chunks.  A left-out file is simply absent
+ *   from images_out and index_out (gnc_png_pack returns GNC_OK for the batch; GNC_UNSUPPORTED is the verdict its
+ *   per-file parser gives internally and never reaches the caller).
+ *   totals[4] = { files in, stream bytes, raw bytes, pixels }.
+ * gnc_png_decode_rgb_u8 (DEVICE): two launches whatever B.  raw: uint8 [raw bytes] scratch; out: uint8 [3 * pixels],
+ *   image j's RGB pixels, row-major, at 3 * pixel_offset; status: int32 [B], 0 = decoded, else the reason, numbered as
+ *   in csrc/inflate.h (a stream zlib would not inflate to exactly raw_bytes with a matching Adler-32, or a filter byte
+ *   > 4) - decode those files with Pillow on the host.  Test status != 0: these codes are their own numbering, not the
+ *   GNC_* return codes (4 there means a bad code-length set).  The device is stricter than Pillow, never laxer. */
+#define GNC_UNSUPPORTED 4                  /* format-neutral name of GNC_JPEG_UNSUPPORTED's value */
+#define GNC_PNG_MAX_RAW_BYTES (2 << 20)   /* one stream inflates at ~5.7 MB/s (DESIGN.md §5 "PNG decode") */
+typedef struct gnc_png_image {
+  int32_t width, height, color_type, bit_depth;
+  int32_t row_bytes;      /* filtered row without its filter byte */
+  int32_t bpp;            /* filter step: bytes per complete pixel, at least 1 */
+  int32_t window;         /* LZ77 window of the zlib header, bytes */
+  int32_t _pad;
+  int64_t stream_offset, stream_bytes;
+  int64_t raw_offset, raw_bytes;
+  int64_t pixel_offset;
+  uint8_t palette[256][3];/* PLTE as Pillow fills it: zero past its end */
+} gnc_png_image_t;
+int gnc_png_pack(const uint8_t* const* datas, const int64_t* sizes, int n, int threads, uint8_t* stream_out,
+                 int64_t stream_capacity, gnc_png_image_t* images_out, int32_t* index_out, int64_t* totals);
+int gnc_png_decode_rgb_u8(const uint8_t* stream, const gnc_png_image_t* images, int B, uint8_t* raw, uint8_t* out,
+                          int32_t* status, gnc_stream_t stream_);
+
 /* Input staging: the resize the reference applies to every image before building its graph,
  *   Image.open(path).convert('RGB').resize((r, r))     utils/image_to_graph/image_to_graph_optimized.py:65-70,
  *                                                      image_to_graph_patch.py / _superpixel.py likewise
